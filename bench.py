@@ -76,6 +76,37 @@ def noise_scale(sigma=SIGMA):
     return int(round(sigma * 2048.0 / std * (1 << 24)))
 
 
+DUMP_LIMIT = 64 << 20               # bytes --dump-outputs writes at most, row indices of sampled arrays included
+
+
+def message_table(rec, nbytes):
+    """Structured message array -> float64 rows (out_sample, buffer_idx, num_bits, the nbytes message bytes)."""
+    import numpy as np
+    t = np.empty((len(rec), 3 + nbytes), dtype=np.float64)
+    t[:, 0] = rec["out_sample"]
+    t[:, 1] = rec["buffer_idx"]
+    t[:, 2] = rec["num_bits"]
+    t[:, 3:] = rec["data"][:, :nbytes]
+    return t
+
+
+def write_outputs(out_dir, arrays):
+    """Each array as out_dir/<name>.npy in float64.  An array with more rows than its equal share of DUMP_LIMIT holds is
+    cut to a fixed, seeded sample of its rows (in order), and the indices of those rows go to <name>_rows.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_LIMIT // len(arrays)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        row_bytes = 8 * (a[0].size if a.ndim > 1 and len(a) else 1)
+        max_rows = share // (row_bytes + 8)
+        if a.ndim > 0 and len(a) > max_rows:
+            rows = np.sort(np.random.default_rng(SEED).choice(len(a), size=max_rows, replace=False))
+            a = a[rows]
+            np.save(os.path.join(out_dir, f"{name}_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 class ClockSampler(threading.Thread):
     """SM clock and throttle reasons during the timed region: NVML polled every 5 ms in-process (the same
     counters `nvidia-smi --query-gpu=clocks.sm,clocks_event_reasons.*` prints; nvidia-smi -lms cannot
@@ -426,7 +457,14 @@ def main():
     ap.add_argument("--e2e-depth", type=int, default=1, help="decodes in flight in the end-to-end (host input) region")
     ap.add_argument("--pipelined-depth", type=int, default=2,
                     help="depth of the extra 'pipelined' measurement (consecutive windows overlapped); 0 = skip it")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float64): messages "
+                         "(rows of out_sample, buffer_idx, num_bits, message bytes); with one GPU also edges (threshold "
+                         "transitions), first_bit, sizes (n_in, n_out, n_buffers) and exit_carry (state, k, num_bits, "
+                         "prev_bit, 32 data bytes).  The inputs are seeded, so two builds can be compared file by file")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -531,6 +569,7 @@ def main():
                 account()
                 last_gpu = g0
         out = last_gpu._result(res)
+        out["exit_carry"] = ex.astuple()
         return out, out["msgs_raw"], acc
 
     def run_steps_multi(iq_arg, n_steps, depth=1, first=first, n=n):
@@ -622,6 +661,16 @@ def main():
     t1 = time.perf_counter()
     dt = t1 - t0
     clocks = sampler.stop(t0, t1)
+
+    if args.dump_outputs and rank == 0:
+        outputs = {"messages": message_table(msgs, dev.nbytes)}
+        if world == 1:
+            # (the handle of the last step still holds its transitions until the next region reuses it)
+            fb, edges = gpus[(args.steps - 1) % depth].edges()
+            state, k, nbits, prev, data = res["exit_carry"]
+            outputs.update(edges=edges, first_bit=[fb], sizes=[res["n_in"], res["n_out"], res["n_buffers"]],
+                           exit_carry=[state, k, nbits, prev] + list(data))
+        write_outputs(args.dump_outputs, outputs)
 
     # ---- extra: the same steps with consecutive decodes overlapped (two handles), as the windows of a long capture
     #      are processed; every step is still a complete decode + stitch inside the timed region ----

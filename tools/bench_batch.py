@@ -1,10 +1,11 @@
 """Independent captures (BASELINE configs[4] shape): N captures x 2^24 samples, devices alternating between
 p3l-nexa2012 and unknown-remote1, filter fs64_fs8, sigma in {0, 0.02, 0.05}, decoded with ookd_gpu_batch_decode
 over H handles per device description.  Prints captures/s and Msamples/s for H = 1, 2, 4 (device-resident input)."""
+import os
 import sys
 import time
 
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import torch
 from ookiedokie_b200 import binding as B, host as H
