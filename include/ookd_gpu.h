@@ -198,6 +198,17 @@ struct ookd_gpu_config {
                                                 screening from then on                                                  */
 #define OOKD_FLAG_NO_SCREEN      2u          /* no screening: the exact tiled kernels compute every output with the
                                                 reference's in-order MACs (same decisions, fp32-issue bound)        */
+/* Capture format.  Neither flag: SC16Q11 (interleaved little-endian int16 I,Q, 4 bytes per sample).  With one of these
+ * the `iq` of ookd_gpu_decode / _decode_shard / _decode_begin / _filtered / ookd_gpu_multi_decode* and
+ * ookd_capture.iq point at BYTES, interleaved I,Q, 2 bytes per sample (pass the byte pointer cast to the declared type);
+ * sample counts, first_sample, halo and output indices stay in samples.  Each 8-bit sample is exactly an SC16Q11 one, so
+ * a decode gives what decoding the widened SC16Q11 capture gives, bit for bit:
+ *   CS8 (HackRF; bladeRF SC8_Q7): int8 k   = k / 128         = SC16Q11 word 16 k
+ *   CU8 (RTL-SDR):                uint8 v  = (v - 127.5)/128 = SC16Q11 word 16 v - 2040
+ * The history before sample 0 and the EOF padding are the value 0 (word 0) in every format.  Both flags together:
+ * ookd_gpu_create returns OOKD_ERR_ARG. */
+#define OOKD_FLAG_INPUT_CS8   1024u
+#define OOKD_FLAG_INPUT_CU8   2048u
 
 struct ookd_gpu_result {
     uint64_t n_in;                           /* input samples consumed incl. EOF zero padding   */
@@ -238,7 +249,8 @@ int  ookd_gpu_create(ookd_gpu **h, const struct ookd_gpu_config *cfg);
 void ookd_gpu_destroy(ookd_gpu *h);
 
 /* Whole-capture decode == running ookiedokie_rx() over a file holding
- * n_samples SC16Q11 samples (interleaved little-endian int16 I,Q): the tail is
+ * n_samples SC16Q11 samples (interleaved little-endian int16 I,Q; with OOKD_FLAG_INPUT_CS8 / _CU8 iq points at
+ * 2-byte samples and the file is their widened SC16Q11 capture): the tail is
  * zero padded to a multiple of samples_per_buffer exactly like
  * sdr_bladerf_file_rx (src/sdr/bladeRF_file.c:106-123).
  * iq may be host memory (pinned recommended; copied in pipelined pieces) or,
@@ -250,7 +262,8 @@ int  ookd_gpu_decode(ookd_gpu *h, const int16_t *iq, uint64_t n_samples,
  * [first_sample, first_sample + n_samples) of a longer capture; first_sample
  * must be a multiple of lcm(samples_per_buffer, total decimation).  iq points
  * at sample first_sample - halo, where halo = ookd_gpu_halo(h) samples of
- * history (fewer only when first_sample < halo: then iq points at sample 0).
+ * history (fewer only when first_sample < halo: then iq points at sample 0); with an 8-bit format flag iq is a byte
+ * pointer, 2 bytes per sample.
  * `last` != 0 applies the EOF zero padding.  entry == NULL starts the state
  * machine in RESET (capture start); otherwise it resumes from *entry, which
  * may be a guess: ookd_gpu_resolve() re-runs only the state machine stage from
@@ -268,7 +281,7 @@ int  ookd_gpu_resolve(ookd_gpu *h, const struct ookd_sm_carry *entry,
  * common case), validates and fills the results.  ookd_gpu_decode_shard is
  * _begin followed by _end.  iq must stay valid until _end returns.  One decode
  * per handle can be in flight; decodes on different handles overlap on the
- * device. */
+ * device.  iq as for ookd_gpu_decode_shard (bytes with an 8-bit format flag). */
 int  ookd_gpu_decode_begin(ookd_gpu *h, const int16_t *iq, int iq_is_device_ptr,
                            uint64_t first_sample, uint64_t n_samples, int last,
                            const struct ookd_sm_carry *entry);
@@ -285,7 +298,7 @@ int  ookd_gpu_decode_end(ookd_gpu *h, struct ookd_sm_carry *exit_, struct ookd_g
  * of messages.  results (nullable) receives per-capture statistics (its msgs
  * pointers are NULL). */
 struct ookd_capture {
-    const int16_t *iq;
+    const int16_t *iq;                       /* in the format of handles[handle] (bytes for CS8 / CU8) */
     uint64_t n_samples;
     int32_t  iq_is_device_ptr;
     uint32_t handle;                         /* index into handles[]                   */
@@ -303,7 +316,8 @@ int  ookd_gpu_batch_decode(ookd_gpu *const *handles, uint32_t n_handles,
  * The result is what ookiedokie_rx()'s loop (src/ookiedokie.c:238-290) prints for the window.
  * iq: host memory pointing at sample first_sample - min(ookd_gpu_multi_halo(), first_sample) (pinned recommended), or,
  * with iq_is_device_ptrs != 0, an array of n_gpus device pointers (const int16_t *const *), pointer g on GPU
- * gpu_ids[g] pointing at shard g's first sample (ookd_gpu_multi_shard_range) minus min(halo, that sample). */
+ * gpu_ids[g] pointing at shard g's first sample (ookd_gpu_multi_shard_range) minus min(halo, that sample).  Offsets are
+ * in samples of the configuration's format (2 bytes each with OOKD_FLAG_INPUT_CS8 / _CU8). */
 typedef struct ookd_gpu_multi ookd_gpu_multi;
 int  ookd_gpu_multi_create(ookd_gpu_multi **m, const struct ookd_gpu_config *cfg /* device_id ignored */,
                            const int32_t *gpu_ids, uint32_t n_gpus);
@@ -332,6 +346,7 @@ int  ookd_gpu_multi_resolve(ookd_gpu_multi *m, const struct ookd_sm_carry *entry
 int  ookd_gpu_multi_edges(ookd_gpu_multi *m, const uint64_t **edges, uint64_t *n_edges, uint32_t *first_bit);
 
 uint32_t ookd_gpu_halo(const ookd_gpu *h);               /* input samples of FIR history  */
+uint32_t ookd_gpu_input_bytes(const ookd_gpu *h);        /* bytes per input sample: 4 (SC16Q11) or 2 (CS8, CU8) */
 uint32_t ookd_gpu_total_decimation(const ookd_gpu *h);
 void ookd_gpu_initial_carry(const ookd_gpu *h, struct ookd_sm_carry *c);  /* RESET, k=0 */
 
@@ -346,7 +361,7 @@ int  ookd_gpu_bits(ookd_gpu *h, uint8_t *bits_out, uint64_t max_out, uint64_t *n
 /* Filtered + decimated samples (interleaved float re,im) computed with the
  * reference's exact in-order fp32 arithmetic (src/fir.c:313-318); the parity
  * dump for fir_filter_and_decimate.  Runs its own kernels; does not disturb
- * the last decode's results. */
+ * the last decode's results.  iq in the handle's format (bytes for CS8 / CU8). */
 int  ookd_gpu_filtered(ookd_gpu *h, const int16_t *iq, uint64_t n_samples, int iq_is_device_ptr,
                        float *out_iq_host, uint64_t max_out, uint64_t *n_out);
 

@@ -27,6 +27,11 @@ FLAG_NO_GRAPH = 64
 FLAG_FUSED_SM = 128
 FLAG_FMA_SCREEN = 256
 FLAG_NO_ADAPTIVE = 512
+FLAG_INPUT_CS8 = 1024
+FLAG_INPUT_CU8 = 2048
+
+# input_format -> (ookd_gpu_config.flags bit, numpy dtype of a host capture); every format is interleaved I,Q
+INPUT_FORMATS = {"sc16q11": (0, np.int16), "cs8": (FLAG_INPUT_CS8, np.int8), "cu8": (FLAG_INPUT_CU8, np.uint8)}
 
 # every symbol include/ookd_gpu.h declares
 EXPORTS = [
@@ -34,7 +39,7 @@ EXPORTS = [
     "ookd_gpu_device_count", "ookd_gpu_strerror", "ookd_gpu_last_error",
     "ookd_gpu_create", "ookd_gpu_destroy", "ookd_gpu_decode", "ookd_gpu_decode_shard",
     "ookd_gpu_decode_begin", "ookd_gpu_decode_end", "ookd_gpu_batch_decode",
-    "ookd_gpu_resolve", "ookd_gpu_halo", "ookd_gpu_total_decimation", "ookd_gpu_initial_carry",
+    "ookd_gpu_resolve", "ookd_gpu_halo", "ookd_gpu_input_bytes", "ookd_gpu_total_decimation", "ookd_gpu_initial_carry",
     "ookd_gpu_edges", "ookd_gpu_bits", "ookd_gpu_filtered", "ookd_gpu_filter_cf", "ookd_gpu_synth", "ookd_gpu_synth_ex",
     "ookd_gpu_host_alloc", "ookd_gpu_host_free", "ookd_gpu_dev_alloc", "ookd_gpu_dev_free",
     "ookd_gpu_memcpy_h2d", "ookd_gpu_memcpy_d2h", "ookd_gpu_filtered_sc16q11",
@@ -185,6 +190,8 @@ def lib():
         L.ookd_gpu_halo.restype = C.c_uint32
         L.ookd_gpu_halo.argtypes = [C.c_void_p]
         L.ookd_gpu_total_decimation.restype = C.c_uint32
+        L.ookd_gpu_input_bytes.argtypes = [C.c_void_p]
+        L.ookd_gpu_input_bytes.restype = C.c_uint32
         L.ookd_gpu_total_decimation.argtypes = [C.c_void_p]
         L.ookd_gpu_initial_carry.argtypes = [C.c_void_p, C.POINTER(SmCarry)]
         L.ookd_gpu_edges.restype = C.c_int
@@ -325,19 +332,46 @@ def device_count():
     return int(lib().ookd_gpu_device_count())
 
 
-def _as_ptr(iq):
-    """numpy int16 array -> (pointer, n_samples, is_device=0, keepalive); (int ptr, n) tuples pass through as device."""
+def _input_format(input_format, flags=0):
+    """input_format name -> (flag, numpy dtype).  The format is chosen by name only: format bits in `flags` would make
+    the handle read bytes while this binding still passed int16 arrays."""
+    if flags & (FLAG_INPUT_CS8 | FLAG_INPUT_CU8):
+        raise ValueError("choose the capture format with input_format=, not with the OOKD_FLAG_INPUT_* bits in flags")
+    if input_format not in INPUT_FORMATS:
+        raise ValueError(f"input_format must be one of {sorted(INPUT_FORMATS)}, not {input_format!r}")
+    return INPUT_FORMATS[input_format]
+
+
+def _host_iq(iq, input_format="sc16q11"):
+    """Host capture -> flat contiguous array of the format's dtype (I, Q interleaved; shape (n, 2) or flat).
+    8-bit captures must already have their dtype (int8 for cs8, uint8 for cu8): converting values between formats is
+    not a cast, so any other dtype -- and an 8-bit array handed to an SC16Q11 handle -- is a ValueError."""
+    dtype = _input_format(input_format)[1]
+    got = getattr(iq, "dtype", None)
+    if input_format != "sc16q11" and got != dtype:
+        raise ValueError(f"a {input_format} capture is a numpy {np.dtype(dtype).name} array, not {got}")
+    if input_format == "sc16q11" and got in (np.dtype(np.int8), np.dtype(np.uint8)):
+        raise ValueError(f"a {got} array is an 8-bit capture: decode it with a handle created with input_format="
+                         f"{'cs8' if got == np.dtype(np.int8) else 'cu8'!r}")
+    return np.ascontiguousarray(iq, dtype=dtype).reshape(-1)
+
+
+def _as_ptr(iq, input_format="sc16q11"):
+    """numpy capture -> (pointer, n_samples, is_device=0, keepalive); (int ptr, n) tuples pass through as device."""
     if isinstance(iq, tuple):
         return C.c_void_p(int(iq[0])), int(iq[1]), 1, None
-    a = np.ascontiguousarray(iq, dtype=np.int16).reshape(-1)
+    a = _host_iq(iq, input_format)
     return C.c_void_p(a.ctypes.data), a.size // 2, 0, a
 
 
 class Gpu:
-    """One ookd_gpu handle."""
+    """One ookd_gpu handle.  input_format: "sc16q11" (int16 I,Q), "cs8" (int8 I,Q) or "cu8" (uint8 I,Q) host arrays;
+    an 8-bit capture decodes exactly as its widened SC16Q11 capture does (include/ookd_gpu.h, OOKD_FLAG_INPUT_*)."""
 
     def __init__(self, filter_stages=None, sm=None, threshold=0.1, samples_per_buffer=8192, device_id=-1,
-                 flags=0, sm_chunk_buffers=0, sm_warmup=0, sm_burst_rounds=0, sub_windows=0):
+                 flags=0, sm_chunk_buffers=0, sm_warmup=0, sm_burst_rounds=0, sub_windows=0, input_format="sc16q11"):
+        flags |= _input_format(input_format, flags)[0]
+        self.input_format = input_format
         L = lib()
         cfg = GpuConfig()
         self._keep = []
@@ -406,8 +440,8 @@ class Gpu:
         return int(lib().ookd_gpu_total_decimation(self.h))
 
     def decode(self, iq):
-        """iq: numpy int16 (host) or (device_ptr, n_samples)."""
-        p, n, is_dev, keep = _as_ptr(iq)
+        """iq: numpy array of the handle's input format (host) or (device_ptr, n_samples)."""
+        p, n, is_dev, keep = _as_ptr(iq, self.input_format)
         res = GpuResult()
         self._check(lib().ookd_gpu_decode(self.h, p, n, is_dev, C.byref(res)), "ookd_gpu_decode")
         return self._result(res)
@@ -417,7 +451,7 @@ class Gpu:
         if isinstance(iq, tuple):
             p, is_dev, keep = C.c_void_p(int(iq[0])), 1, None
         else:
-            keep = np.ascontiguousarray(iq, dtype=np.int16).reshape(-1)
+            keep = _host_iq(iq, self.input_format)
             p, is_dev = C.c_void_p(keep.ctypes.data), 0
         res = GpuResult()
         ex = SmCarry()
@@ -432,7 +466,7 @@ class Gpu:
         if isinstance(iq, tuple):
             p, is_dev, keep = C.c_void_p(int(iq[0])), 1, None
         else:
-            keep = np.ascontiguousarray(iq, dtype=np.int16).reshape(-1)
+            keep = _host_iq(iq, self.input_format)
             p, is_dev = C.c_void_p(keep.ctypes.data), 0
         self._keep = keep
         en = SmCarry.fromtuple(entry) if entry is not None else None
@@ -470,7 +504,7 @@ class Gpu:
         return out
 
     def filtered(self, iq):
-        p, n, is_dev, keep = _as_ptr(iq)
+        p, n, is_dev, keep = _as_ptr(iq, self.input_format)
         m = C.c_uint64()
         self._check(lib().ookd_gpu_filtered(self.h, p, n, is_dev, None, 0, C.byref(m)), "ookd_gpu_filtered")
         out = np.empty((m.value, 2), dtype=np.float32)
@@ -501,7 +535,9 @@ class MultiGpu:
     """One ookd_gpu_multi handle: a window time-sharded over several GPUs of this process."""
 
     def __init__(self, gpu_ids, filter_stages=None, sm=None, threshold=0.1, samples_per_buffer=8192, flags=0,
-                 sm_chunk_buffers=0):
+                 sm_chunk_buffers=0, input_format="sc16q11"):
+        flags |= _input_format(input_format, flags)[0]
+        self.input_format = input_format
         L = lib()
         cfg = GpuConfig()
         self._keep = []
@@ -545,13 +581,13 @@ class MultiGpu:
         return int(a.value), int(b.value)
 
     def decode(self, iq, first_sample=0, n_samples=None, last=True, entry=None, device_ptrs=None):
-        """iq: numpy int16 host array starting at sample first_sample - min(halo, first_sample); or device_ptrs:
+        """iq: numpy host array (the handle's input format) starting at sample first_sample - min(halo, first_sample); or device_ptrs:
         list of per-GPU device pointers.  -> (result dict, exit carry tuple)."""
         if device_ptrs is not None:
             arr = (C.c_void_p * len(device_ptrs))(*[int(p) for p in device_ptrs])
             p, is_dev, keep = C.cast(arr, C.c_void_p), 1, arr
         else:
-            keep = np.ascontiguousarray(iq, dtype=np.int16).reshape(-1)
+            keep = _host_iq(iq, self.input_format)
             p, is_dev = C.c_void_p(keep.ctypes.data), 0
             if n_samples is None:
                 n_samples = keep.size // 2 - min(self.halo, first_sample)
@@ -605,7 +641,7 @@ def synth(n_samples, toggles, i_on, q_on, noise_scale, seed, first_sample=0, dev
 
 def batch_decode(gpus, captures, msgs_cap=None):
     """Independent captures through ookd_gpu_batch_decode.  gpus: list of Gpu handles; captures: list of
-    (iq, handle_index) with iq a numpy int16 array (host) or (device_ptr, n_samples).
+    (iq, handle_index) with iq a numpy array in the input format of gpus[handle_index] (host) or (device_ptr, n_samples).
     -> list of structured message arrays (MSG_DTYPE), one per capture, plus the per-capture statistics."""
     n = len(captures)
     caps = (Capture * max(n, 1))()
@@ -614,7 +650,7 @@ def batch_decode(gpus, captures, msgs_cap=None):
         if isinstance(iq, tuple):
             caps[i].iq, caps[i].n_samples, caps[i].iq_is_device_ptr = int(iq[0]), int(iq[1]), 1
         else:
-            a = np.ascontiguousarray(iq, dtype=np.int16).reshape(-1)
+            a = _host_iq(iq, gpus[hi].input_format)
             keep.append(a)
             caps[i].iq, caps[i].n_samples, caps[i].iq_is_device_ptr = a.ctypes.data, a.size // 2, 0
         caps[i].handle = hi

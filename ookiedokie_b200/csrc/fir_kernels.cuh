@@ -16,7 +16,7 @@
 
 #include <climits>
 
-#include "ookd_common.cuh"
+#include "input_fmt.cuh"
 
 namespace ookd {
 
@@ -26,7 +26,7 @@ namespace ookd {
 //    shapes without a tiled kernel.  One thread per output, taps staged in shared memory.
 // =======================================================================================
 struct GenericStageArgs {
-    const void *in;          // int16x2 words (IN_I16) or float2
+    const void *in;          // the capture (IN_I16, format FMT: input_fmt.cuh) or float2
     i64  in_base;            // global index of in[0]
     i64  in_valid_end;       // inputs >= this index read as zero
     const float *taps;       // device, T floats
@@ -38,7 +38,7 @@ struct GenericStageArgs {
     float pstar;
 };
 
-template <bool IN_I16>
+template <bool IN_I16, int FMT>
 __global__ void __launch_bounds__(256) fir_stage_generic_kernel(const GenericStageArgs a)
 {
     extern __shared__ float s_taps[];
@@ -57,7 +57,11 @@ __global__ void __launch_bounds__(256) fir_stage_generic_kernel(const GenericSta
             float2 x = make_float2(0.0f, 0.0f);
             if (g >= 0 && g < a.in_valid_end) {
                 if (IN_I16) {
-                    x = sc16q11_to_float2(((const uint32_t *) a.in)[g - a.in_base]);
+                    if constexpr (FMT == FMT_SC16Q11) {     // (a plain load, not __ldg: its SASS is kept as it was)
+                        x = sc16q11_to_float2(((const uint32_t *) a.in)[g - a.in_base]);
+                    } else {
+                        x = sc16q11_to_float2(load_word<FMT>((const uint32_t *) a.in, g - a.in_base));
+                    }
                 } else {
                     x = ((const float2 *) a.in)[g - a.in_base];
                 }
@@ -96,8 +100,8 @@ struct TapsParam {
 };
 
 struct TiledArgs {
-    const uint32_t *in;      // int16x2 words
-    i64  in_base;            // global index of in[0]; (tile input start - in_base) 16B-aligned or scalar path
+    const uint32_t *in;      // the capture, in the kernel's input format (input_fmt.cuh)
+    i64  in_base;            // global index of sample 0 of in; (tile input start - in_base) 16B-aligned or scalar path
     i64  in_valid_end;
     i64  out_lo, out_hi;     // global output range; out_lo % (256*R) == 0 relative to bit_base rule below
     uint8_t *out_bits;       // packed decisions (bytes)
@@ -138,6 +142,7 @@ struct ScreenArgs {
 // K0; on an OOK capture most windows are silence, so if even the silence is above K0 (noise floor too high) they decide
 // almost nothing and every group would go to the exact kernel.  256 windows spread over the capture are enough to tell:
 // fewer than 40 % provably off => FMA screening.  One small CTA, no host round trip (the FIR kernels read the verdict).
+template <int FMT>
 __global__ void __launch_bounds__(1024) screen_probe_kernel(const TiledArgs a, int dec, int window, uint32_t k0, uint32_t *mode)
 {
     // 32 warps x 8 windows; lane i of a warp reads samples i, i + 32, ... of the window (coalesced)
@@ -152,7 +157,7 @@ __global__ void __launch_bounds__(1024) screen_probe_kernel(const TiledArgs a, i
         unsigned long long e = 0;
         for (int i = (int) lane; i < window; i += 32) {
             const i64 g = newest - i;
-            const uint32_t w = (g >= 0 && g >= a.in_base && g < a.in_valid_end) ? __ldg(a.in + (g - a.in_base)) : 0u;
+            const uint32_t w = (g >= 0 && g >= a.in_base && g < a.in_valid_end) ? load_word<FMT>(a.in, g - a.in_base) : 0u;
             const long long I = (short) (w & 0xFFFFu), Q = ((int) w) >> 16;
             e += (unsigned long long) (I * I + Q * Q);
         }
@@ -208,7 +213,7 @@ __device__ __forceinline__ uint32_t fma_classify(float re, float im, float hi2, 
     return (p >= hi2) ? 1u : ((p < lo2) ? 0u : 2u);
 }
 
-template <int T, int R, bool FMA, bool ADAPT>
+template <int T, int R, bool FMA, bool ADAPT, int FMT>
 __global__ void __launch_bounds__(256, 2)
 fir1_tiled_kernel(const ScreenArgs sa, const TapsParam<T> taps, const FmaBand band)
 {
@@ -238,25 +243,27 @@ fir1_tiled_kernel(const ScreenArgs sa, const TapsParam<T> taps, const FmaBand ba
         const i64 o0 = a.out_lo + (i64) tile * L;     // first output of the tile
         const i64 g0 = o0 - HALO;                     // first staged input
 
-        // ---- stage inputs: 4 samples (16 B) per thread per step ----
-        const bool aligned = (((g0 - a.in_base) & 3) == 0) && ((((uintptr_t) a.in) & 15) == 0);
+        // ---- stage inputs: VS samples (16 B) per thread per step; the vector load needs the byte offset of sample g0
+        //      (a multiple of VS samples from in_base) and the pointer 16-byte aligned ----
+        constexpr int VS = in_vec<FMT>();
+        static_assert(NS % VS == 0, "whole vectors");
+        const bool aligned = (((g0 - a.in_base) & (VS - 1)) == 0) && ((((uintptr_t) a.in) & 15) == 0);
         float m2 = 0.0f;
-        for (int q = threadIdx.x; q < NS / 4; q += NT) {
-            const i64 g = g0 + 4 * q;
-            uint32_t w[4];
-            if (aligned && g >= a.in_base && g >= 0 && g + 4 <= a.in_valid_end) {
-                const uint4 v = __ldg((const uint4 *) (a.in + (g - a.in_base)));
-                w[0] = v.x; w[1] = v.y; w[2] = v.z; w[3] = v.w;
+        for (int q = threadIdx.x; q < NS / VS; q += NT) {
+            const i64 g = g0 + VS * q;
+            uint32_t w[VS];
+            if (aligned && g >= a.in_base && g >= 0 && g + VS <= a.in_valid_end) {
+                load_words16<FMT>(a.in, g - a.in_base, w);
             } else {
 #pragma unroll
-                for (int e = 0; e < 4; e++) {
+                for (int e = 0; e < VS; e++) {
                     const i64 ge = g + e;
-                    w[e] = (ge >= 0 && ge >= a.in_base && ge < a.in_valid_end) ? __ldg(a.in + (ge - a.in_base)) : 0u;
+                    w[e] = (ge >= 0 && ge >= a.in_base && ge < a.in_valid_end) ? load_word<FMT>(a.in, ge - a.in_base) : 0u;
                 }
             }
 #pragma unroll
-            for (int e = 0; e < 4; e++) {
-                const int s = 4 * q + e;
+            for (int e = 0; e < VS; e++) {
+                const int s = VS * q + e;
                 const float2 x = sc16q11_to_float2(w[e]);
                 s_x[s + (s >> LOGR)] = x;
                 if constexpr (FMA) m2 = fmaxf(m2, fmaf(x.x, x.x, x.y * x.y));
@@ -376,7 +383,7 @@ fir1_tiled_kernel(const ScreenArgs sa, const TapsParam<T> taps, const FmaBand ba
 // Exact recomputation of the groups the screen left undecided: one THREAD per group of 8 outputs.  The 39 samples the
 // group's windows cover are read once (ten 16-byte loads when the input is 16-byte aligned), converted once and kept in
 // registers; 8 outputs = 16 independent exact accumulator chains per thread.
-template <int T>
+template <int T, int FMT>
 __global__ void __launch_bounds__(128) fir1_refine_group_kernel(const ScreenArgs sa, const TapsParam<T> taps)
 {
     static_assert(T == 32, "window of 8 outputs = 39 samples, fetched as 40");
@@ -388,21 +395,20 @@ __global__ void __launch_bounds__(128) fir1_refine_group_kernel(const ScreenArgs
         const i64 n0 = a.bit_base + (i64) grp * 8;             // first output of the group
         const i64 g0 = n0 - T;                                 // first sample fetched (one more than needed)
         float2 win[T + 8];
-        if (ptr_ok && (((g0 - a.in_base) & 3) == 0) && g0 >= a.in_base && g0 >= 0 && g0 + (T + 8) <= a.in_valid_end) {
-            const uint4 *src = (const uint4 *) (a.in + (g0 - a.in_base));
+        constexpr int VS = in_vec<FMT>();                      // 16-byte loads: byte offset of g0 a multiple of 16
+        if (ptr_ok && (((g0 - a.in_base) & (VS - 1)) == 0) && g0 >= a.in_base && g0 >= 0 && g0 + (T + 8) <= a.in_valid_end) {
 #pragma unroll
-            for (int v = 0; v < (T + 8) / 4; v++) {
-                const uint4 x = __ldg(src + v);
-                win[4 * v] = sc16q11_to_float2(x.x);
-                win[4 * v + 1] = sc16q11_to_float2(x.y);
-                win[4 * v + 2] = sc16q11_to_float2(x.z);
-                win[4 * v + 3] = sc16q11_to_float2(x.w);
+            for (int v = 0; v < (T + 8) / VS; v++) {
+                uint32_t x[VS];
+                load_words16<FMT>(a.in, (g0 - a.in_base) + VS * v, x);
+#pragma unroll
+                for (int e = 0; e < VS; e++) win[VS * v + e] = sc16q11_to_float2(x[e]);
             }
         } else {
 #pragma unroll
             for (int q = 0; q < T + 8; q++) {
                 const i64 g = g0 + q;
-                win[q] = sc16q11_to_float2((g >= 0 && g >= a.in_base && g < a.in_valid_end) ? __ldg(a.in + (g - a.in_base)) : 0u);
+                win[q] = sc16q11_to_float2((g >= 0 && g >= a.in_base && g < a.in_valid_end) ? load_word<FMT>(a.in, g - a.in_base) : 0u);
             }
         }
         float re[8], im[8];
@@ -457,7 +463,7 @@ struct Taps2Param {
 // ~77 instructions per input sample against the 64 the arithmetic itself needs.
 constexpr int F2X_NT = 288, F2X_M = 512, F2X_IN = 4 * F2X_M + 80, F2X_NS = 2 * F2X_M + 30;
 
-template <bool FMA, bool ADAPT>
+template <bool FMA, bool ADAPT, int FMT>
 __global__ void __launch_bounds__(F2X_NT, 2) fir2_tiled_kernel(const ScreenArgs sa, const Taps2Param taps, const FmaBand band)
 {
     __shared__ float2 s_x[F2X_IN + F2X_IN / 8 + 8];        // (+8: the last phase-1 thread reads a few slots past its valid window)
@@ -471,25 +477,26 @@ __global__ void __launch_bounds__(F2X_NT, 2) fir2_tiled_kernel(const ScreenArgs 
     const i64 m0 = a.out_lo + (i64) blockIdx.x * F2X_M;       // first output of the tile (a.out_lo % 8 == a.bit_base % 8)
     const i64 g0 = 4 * m0 - 80;                               // first staged input
 
-    // ---- stage inputs: 4 samples (16 B) per thread per step ----
-    const bool aligned = (((g0 - a.in_base) & 3) == 0) && ((((uintptr_t) a.in) & 15) == 0);
+    // ---- stage inputs: VS samples (16 B) per thread per step (alignment as in fir1_tiled_kernel) ----
+    constexpr int VS = in_vec<FMT>();
+    static_assert(F2X_IN % VS == 0, "whole vectors");
+    const bool aligned = (((g0 - a.in_base) & (VS - 1)) == 0) && ((((uintptr_t) a.in) & 15) == 0);
     float m2 = 0.0f;
-    for (int q = t; q < F2X_IN / 4; q += F2X_NT) {
-        const i64 g = g0 + 4 * q;
-        uint32_t w[4];
-        if (aligned && g >= a.in_base && g >= 0 && g + 4 <= a.in_valid_end) {
-            const uint4 v = __ldg((const uint4 *) (a.in + (g - a.in_base)));
-            w[0] = v.x; w[1] = v.y; w[2] = v.z; w[3] = v.w;
+    for (int q = t; q < F2X_IN / VS; q += F2X_NT) {
+        const i64 g = g0 + VS * q;
+        uint32_t w[VS];
+        if (aligned && g >= a.in_base && g >= 0 && g + VS <= a.in_valid_end) {
+            load_words16<FMT>(a.in, g - a.in_base, w);
         } else {
 #pragma unroll
-            for (int e = 0; e < 4; e++) {
+            for (int e = 0; e < VS; e++) {
                 const i64 ge = g + e;
-                w[e] = (ge >= 0 && ge >= a.in_base && ge < a.in_valid_end) ? __ldg(a.in + (ge - a.in_base)) : 0u;
+                w[e] = (ge >= 0 && ge >= a.in_base && ge < a.in_valid_end) ? load_word<FMT>(a.in, ge - a.in_base) : 0u;
             }
         }
 #pragma unroll
-        for (int e = 0; e < 4; e++) {
-            const int x = 4 * q + e;
+        for (int e = 0; e < VS; e++) {
+            const int x = VS * q + e;
             const float2 v = sc16q11_to_float2(w[e]);
             s_x[x + (x >> 3)] = v;
             if constexpr (FMA) m2 = fmaxf(m2, fmaf(v.x, v.x, v.y * v.y));
@@ -600,6 +607,7 @@ __global__ void __launch_bounds__(F2X_NT, 2) fir2_tiled_kernel(const ScreenArgs 
 // inputs per step) and fed to every output y[m] they belong to: walking u downwards visits the taps of each y[m] in
 // the reference's order j = 0, 1, ... (src/fir.c:313-318), so all sums stay bit-exact; 4.4x fewer MACs than the
 // lane-per-output form.
+template <int FMT>
 __global__ void __launch_bounds__(128) fir2_refine_group_kernel(const ScreenArgs sa, const Taps2Param taps)
 {
     const TiledArgs &a = sa.t;
@@ -612,8 +620,8 @@ __global__ void __launch_bounds__(128) fir2_refine_group_kernel(const ScreenArgs
         const i64 g_bot = 2 * (u_top - 45) + 1 - 15;           // oldest input: 4 m0 - 74
         const bool inside = g_bot >= a.in_base && g_bot >= 0 && g_top < a.in_valid_end;
         auto sample = [&](i64 g) -> float2 {
-            if (inside) return sc16q11_to_float2(__ldg(a.in + (g - a.in_base)));
-            return sc16q11_to_float2((g >= 0 && g >= a.in_base && g < a.in_valid_end) ? __ldg(a.in + (g - a.in_base)) : 0u);
+            if (inside) return sc16q11_to_float2(load_word<FMT>(a.in, g - a.in_base));
+            return sc16q11_to_float2((g >= 0 && g >= a.in_base && g < a.in_valid_end) ? load_word<FMT>(a.in, g - a.in_base) : 0u);
         };
         float2 w[16];                                          // w[k] = x[2u+1-k] for the current u
 #pragma unroll

@@ -14,6 +14,7 @@
 #include <algorithm>
 #include <cstring>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "ookd_common.cuh"
@@ -64,6 +65,8 @@ struct ookd_gpu {
     uint32_t burst_rounds = 1;
     bool burst_fixed = false;         // sm_burst_rounds given in the configuration: no adaptation
     uint32_t flags = 0;
+    int fmt = FMT_SC16Q11;            // capture format (OOKD_FLAG_INPUT_*, input_fmt.cuh)
+    uint32_t in_bytes = 4;            // ... its bytes per sample
     bool screen = false;
     bool screen2 = false;             // dec4 shape: screen + refine (else the exact tiled two-stage kernel)
     bool fma = false;                 // FMA screening (fused multiply-add pass + rigorous band, exact refine of the band):
@@ -328,12 +331,31 @@ encode_tiled_fn tensor_map_encoder()
     return fn;
 }
 
+// Calls f(std::integral_constant<int, FMT>) for the handle's capture format: every kernel that reads the capture is
+// instantiated per format (input_fmt.cuh).
+template <typename F>
+void with_fmt(int fmt, F &&f)
+{
+    if (fmt == FMT_CS8) {
+        f(std::integral_constant<int, FMT_CS8>());
+    } else if (fmt == FMT_CU8) {
+        f(std::integral_constant<int, FMT_CU8>());
+    } else {
+        f(std::integral_constant<int, FMT_SC16Q11>());
+    }
+}
+
 typedef void (*screen_tma_kernel_t)(const CUtensorMap, const ScreenTmaArgs, const ScreenParams);
 
-screen_tma_kernel_t screen_tma_fn(int dec, bool adapt)
+screen_tma_kernel_t screen_tma_fn(int dec, bool adapt, int fmt)
 {
-    if (dec == 1) return adapt ? fir_screen_tma_kernel<1, true> : fir_screen_tma_kernel<1, false>;
-    return adapt ? fir_screen_tma_kernel<4, true> : fir_screen_tma_kernel<4, false>;
+    screen_tma_kernel_t k = nullptr;
+    with_fmt(fmt, [&](auto fc) {
+        constexpr int FMT = decltype(fc)::value;
+        if (dec == 1) k = adapt ? fir_screen_tma_kernel<1, true, FMT> : fir_screen_tma_kernel<1, false, FMT>;
+        else k = adapt ? fir_screen_tma_kernel<4, true, FMT> : fir_screen_tma_kernel<4, false, FMT>;
+    });
+    return k;
 }
 
 // OOKD_FLAG_SHARE_SMS: the persistent screening kernels of different handles on one device must not overlap
@@ -380,23 +402,26 @@ ScreenArgs screen_args(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_va
 int launch_screen_tma(ookd_gpu *h, const ScreenArgs &sa, const ScreenParams &sp, const uint32_t *d_in, i64 in_base,
                       i64 in_valid_end, u64 tiles, int dec)
 {
-    // Tensor view: rows of 32 samples starting at row0 (the first input of a tile of this decode, at or after the
-    // first sample present); only tiles that lie wholly inside complete rows use the copy engine.
+    // Tensor view: rows of 128 bytes (32 words = 32 SC16Q11 samples or 64 8-bit samples) starting at row0 (the first
+    // input of a tile of this decode, at or after the first sample present); only tiles that lie wholly inside
+    // complete rows use the copy engine.
     ScreenTmaArgs ta{};
     ta.s = sa;
+    const i64 rs = 128 / h->in_bytes;                         // samples per row
     const i64 first_present = in_base > 0 ? in_base : 0;
     i64 row0 = h->bit_base * dec;
     if (row0 < first_present) row0 += (first_present - row0 + STMA_L - 1) / STMA_L * STMA_L;
-    const uintptr_t addr0 = (uintptr_t) (d_in + (row0 - in_base));
-    const i64 n_rows = (in_valid_end - row0) / 32;
+    const uintptr_t addr0 = (uintptr_t) d_in + (uintptr_t) ((row0 - in_base) * h->in_bytes);
+    const i64 n_rows = (in_valid_end - row0) / rs;
     CUtensorMap tmap;
     memset(&tmap, 0, sizeof(tmap));
-    bool ok = (addr0 % 16 == 0) && n_rows >= STMA_L / 32 && n_rows < (1ll << 31) && tensor_map_encoder() &&
+    bool ok = (addr0 % 16 == 0) && n_rows >= STMA_L / rs && n_rows < (1ll << 31) && tensor_map_encoder() &&
               !(h->flags & OOKD_FLAG_NO_TMA);
     if (ok) {
         const cuuint64_t gdim[2] = {32, (cuuint64_t) n_rows};
         const cuuint64_t gstride[1] = {128};
-        const cuuint32_t box[2] = {32, STMA_L / 32};
+        // SC16Q11: one copy per tile; 8-bit: one copy per warp (screen_tma.cuh)
+        const cuuint32_t box[2] = {32, (cuuint32_t) (h->in_bytes == 4 ? STMA_L / rs : STMA8_BOX_ROWS)};
         const cuuint32_t estr[2] = {1, 1};
         ok = tensor_map_encoder()(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT32, 2, (void *) addr0, gdim, gstride, box, estr,
                                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
@@ -405,7 +430,7 @@ int launch_screen_tma(ookd_gpu *h, const ScreenArgs &sa, const ScreenParams &sp,
     ta.row0_sample = row0;
     if (ok) {
         ta.fast_lo = (uint32_t) ((row0 - h->bit_base * dec) / STMA_L);
-        ta.fast_hi = (uint32_t) ((row0 + n_rows * 32 - h->bit_base * dec) / STMA_L);
+        ta.fast_hi = (uint32_t) ((row0 + n_rows * rs - h->bit_base * dec) / STMA_L);
     } else {
         ta.fast_lo = ta.fast_hi = 0;
     }
@@ -417,7 +442,7 @@ int launch_screen_tma(ookd_gpu *h, const ScreenArgs &sa, const ScreenParams &sp,
     cudaEvent_t *tok = (share && use_token) ? screen_token(h->device) : nullptr;
     if (tok) CU(h, cudaStreamWaitEvent(h->s_compute, *tok, 0));
     const unsigned grid = (unsigned) (tiles < ctas ? tiles : ctas);
-    screen_tma_fn(dec, h->adaptive)<<<grid, STMA_NT, STMA_SMEM_BYTES, h->s_compute>>>(tmap, ta, sp);
+    screen_tma_fn(dec, h->adaptive, h->fmt)<<<grid, STMA_NT, STMA_SMEM_BYTES, h->s_compute>>>(tmap, ta, sp);
     if (tok) CU(h, cudaEventRecord(*tok, h->s_compute));
     return OOKD_OK;
 }
@@ -447,15 +472,17 @@ int launch_fir(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_valid_end,
             FmaBand band{};
             if (h->adaptive) h->launches++;
             // (adaptive decodes are short: when the probe did not choose this form its CTAs return at once)
-            if (h->adaptive) {
-                make_fma_band(h, band);
-                fir1_tiled_kernel<32, TILE_R, true, true><<<(unsigned) tiles, 256, 0, h->s_compute>>>(sa, tp, band);
-            } else if (h->fma) {
-                make_fma_band(h, band);
-                fir1_tiled_kernel<32, TILE_R, true, false><<<(unsigned) tiles, 256, 0, h->s_compute>>>(sa, tp, band);
-            } else {
-                fir1_tiled_kernel<32, TILE_R, false, false><<<(unsigned) tiles, 256, 0, h->s_compute>>>(sa, tp, band);
-            }
+            if (h->adaptive || h->fma) make_fma_band(h, band);
+            with_fmt(h->fmt, [&](auto fc) {
+                constexpr int FMT = decltype(fc)::value;
+                if (h->adaptive) {
+                    fir1_tiled_kernel<32, TILE_R, true, true, FMT><<<(unsigned) tiles, 256, 0, h->s_compute>>>(sa, tp, band);
+                } else if (h->fma) {
+                    fir1_tiled_kernel<32, TILE_R, true, false, FMT><<<(unsigned) tiles, 256, 0, h->s_compute>>>(sa, tp, band);
+                } else {
+                    fir1_tiled_kernel<32, TILE_R, false, false, FMT><<<(unsigned) tiles, 256, 0, h->s_compute>>>(sa, tp, band);
+                }
+            });
         }
         h->launches++;
         CU(h, cudaGetLastError());
@@ -485,15 +512,17 @@ int launch_fir(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_valid_end,
         sa.t.out_lo = o_begin; sa.t.out_hi = o_end;
         const u64 tiles = (u64) (o_end - o_begin + F2X_M - 1) / F2X_M;
         FmaBand band{};
-        if (h->adaptive) {
-            make_fma_band(h, band);
-            fir2_tiled_kernel<true, true><<<(unsigned) tiles, F2X_NT, 0, h->s_compute>>>(sa, tp, band);
-        } else if (h->fma) {
-            make_fma_band(h, band);
-            fir2_tiled_kernel<true, false><<<(unsigned) tiles, F2X_NT, 0, h->s_compute>>>(sa, tp, band);
-        } else {
-            fir2_tiled_kernel<false, false><<<(unsigned) tiles, F2X_NT, 0, h->s_compute>>>(sa, tp, band);
-        }
+        if (h->adaptive || h->fma) make_fma_band(h, band);
+        with_fmt(h->fmt, [&](auto fc) {
+            constexpr int FMT = decltype(fc)::value;
+            if (h->adaptive) {
+                fir2_tiled_kernel<true, true, FMT><<<(unsigned) tiles, F2X_NT, 0, h->s_compute>>>(sa, tp, band);
+            } else if (h->fma) {
+                fir2_tiled_kernel<true, false, FMT><<<(unsigned) tiles, F2X_NT, 0, h->s_compute>>>(sa, tp, band);
+            } else {
+                fir2_tiled_kernel<false, false, FMT><<<(unsigned) tiles, F2X_NT, 0, h->s_compute>>>(sa, tp, band);
+            }
+        });
         h->launches++;
         CU(h, cudaGetLastError());
         return OOKD_OK;
@@ -512,7 +541,9 @@ int launch_fir_refine(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_val
         tp.d_t1 = h->stages[0].d_taps;
         tp.d_t2 = h->stages[1].d_taps;
         ScreenArgs sa = screen_args(h, d_in, in_base, in_valid_end);
-        fir2_refine_group_kernel<<<16 * h->n_sm, 128, 0, h->s_compute>>>(sa, tp);
+        with_fmt(h->fmt, [&](auto fc) {
+            fir2_refine_group_kernel<decltype(fc)::value><<<16 * h->n_sm, 128, 0, h->s_compute>>>(sa, tp);
+        });
         h->launches++;
         CU(h, cudaGetLastError());
         return OOKD_OK;
@@ -521,7 +552,9 @@ int launch_fir_refine(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_val
     TapsParam<32> tp;
     memcpy(tp.t, h->stages[0].taps.data(), sizeof(tp.t));
     ScreenArgs sa = screen_args(h, d_in, in_base, in_valid_end);
-    fir1_refine_group_kernel<32><<<16 * h->n_sm, 128, 0, h->s_compute>>>(sa, tp);
+    with_fmt(h->fmt, [&](auto fc) {
+        fir1_refine_group_kernel<32, decltype(fc)::value><<<16 * h->n_sm, 128, 0, h->s_compute>>>(sa, tp);
+    });
     h->launches++;
     CU(h, cudaGetLastError());
     return OOKD_OK;
@@ -543,7 +576,7 @@ int launch_fir_exact_all(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_
 
 // ---- shape-agnostic chain: one launch per stage, intermediates in HBM ----
 // Computes final outputs [o_lo, o_hi); writes decisions (bits != null) and/or the final
-// stage's samples (out_cf != null, out_cf[0] <-> o_lo).  `in` is int16x2 (in_is_i16) or float2.
+// stage's samples (out_cf != null, out_cf[0] <-> o_lo).  `in` is the capture in the handle's format (in_is_i16) or float2.
 int run_generic_chain(ookd_gpu *h, const void *d_in, bool in_is_i16, i64 in_base, i64 in_valid_end,
                       i64 o_lo, i64 o_hi, float2 *out_cf, uint32_t *bits, i64 bit_base)
 {
@@ -583,9 +616,11 @@ int run_generic_chain(ookd_gpu *h, const void *d_in, bool in_is_i16, i64 in_base
         const unsigned grid = (unsigned) ((n + 255) / 256);
         const size_t smem = st.T * sizeof(float);
         if (src_i16) {
-            fir_stage_generic_kernel<true><<<grid, 256, smem, h->s_compute>>>(a);
+            with_fmt(h->fmt, [&](auto fc) {
+                fir_stage_generic_kernel<true, decltype(fc)::value><<<grid, 256, smem, h->s_compute>>>(a);
+            });
         } else {
-            fir_stage_generic_kernel<false><<<grid, 256, smem, h->s_compute>>>(a);
+            fir_stage_generic_kernel<false, FMT_SC16Q11><<<grid, 256, smem, h->s_compute>>>(a);
         }
         h->launches++;
         CU(h, cudaGetLastError());
@@ -1455,6 +1490,7 @@ int ookd_gpu_create(ookd_gpu **out, const struct ookd_gpu_config *cfg)
 {
     if (!out || !cfg || cfg->samples_per_buffer == 0) return OOKD_ERR_ARG;
     *out = nullptr;
+    if ((cfg->flags & OOKD_FLAG_INPUT_CS8) && (cfg->flags & OOKD_FLAG_INPUT_CU8)) return OOKD_ERR_ARG;   // one format
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return OOKD_ERR_CUDA;
     int dev = cfg->device_id;
@@ -1472,6 +1508,8 @@ int ookd_gpu_create(ookd_gpu **out, const struct ookd_gpu_config *cfg)
     h->pstar = ookd_power_threshold(cfg->threshold);
     h->spb = cfg->samples_per_buffer;
     h->flags = cfg->flags;
+    h->fmt = (cfg->flags & OOKD_FLAG_INPUT_CS8) ? FMT_CS8 : (cfg->flags & OOKD_FLAG_INPUT_CU8) ? FMT_CU8 : FMT_SC16Q11;
+    h->in_bytes = h->fmt == FMT_SC16Q11 ? 4 : 2;
     h->chunk_buffers = cfg->sm_chunk_buffers ? cfg->sm_chunk_buffers : 64;
     h->warmup = cfg->sm_warmup != 0 || (cfg->sub_windows > 1 && cfg->sm);
     h->burst_rounds = cfg->sm_burst_rounds ? (cfg->sm_burst_rounds < 16 ? cfg->sm_burst_rounds : 16) : FAST_BURST_ROUNDS;
@@ -1532,8 +1570,10 @@ int ookd_gpu_create(ookd_gpu **out, const struct ookd_gpu_config *cfg)
     }
     h->total_dec = (uint32_t) dec;
     h->halo_fir = (uint32_t) halo;
-    // one extra byte of decisions in front of a shard gives the edge detector its predecessor
-    h->halo = (uint32_t) ((halo + 8 * dec + 3) & ~3ull);
+    // one extra byte of decisions in front of a shard gives the edge detector its predecessor; rounded to 16 bytes of
+    // input (4 SC16Q11 samples, 8 8-bit samples) so that a shard pointer keeps the alignment the vector loads need
+    const u64 halo_round = 16 / h->in_bytes - 1;
+    h->halo = (uint32_t) ((halo + 8 * dec + halo_round) & ~halo_round);
     if (h->warmup && cfg->sm) {
         // the warm-up history is exactly one chunk, and a chunk must be a whole number of lcm(spb, dec) units
         const u64 unit = dec / gcd64(h->spb, dec);
@@ -1563,7 +1603,7 @@ int ookd_gpu_create(ookd_gpu **out, const struct ookd_gpu_config *cfg)
     {
         for (int dec : {1, 4}) {
             for (bool adapt : {false, true}) {
-                if (cudaFuncSetAttribute(screen_tma_fn(dec, adapt), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                if (cudaFuncSetAttribute(screen_tma_fn(dec, adapt, h->fmt), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          STMA_SMEM_BYTES) != cudaSuccess) {
                     cudaGetLastError();
                     CREATE_FAIL(OOKD_ERR_CUDA);
@@ -1629,6 +1669,7 @@ int ookd_gpu_create(ookd_gpu **out, const struct ookd_gpu_config *cfg)
 }
 
 uint32_t ookd_gpu_halo(const ookd_gpu *h) { return h ? h->halo : 0; }
+uint32_t ookd_gpu_input_bytes(const ookd_gpu *h) { return h ? h->in_bytes : 0; }
 uint32_t ookd_gpu_total_decimation(const ookd_gpu *h) { return h ? h->total_dec : 0; }
 
 void ookd_gpu_initial_carry(const ookd_gpu *h, struct ookd_sm_carry *c)
@@ -1717,8 +1758,10 @@ int ookd_gpu_decode_begin(ookd_gpu *h, const int16_t *iq, int iq_is_device_ptr, 
         TiledArgs pa{};
         pa.in = d_src; pa.in_base = in_base; pa.in_valid_end = in_valid_end;
         pa.out_lo = h->bit_base; pa.out_hi = o_hi_probe;
-        screen_probe_kernel<<<1, 1024, 0, h->s_compute>>>(pa, (int) h->total_dec, (int) h->halo_fir + 1, sp.k0,
-                                                         (uint32_t *) ((char *) h->scalars.p + 344));
+        with_fmt(h->fmt, [&](auto fc) {
+            screen_probe_kernel<decltype(fc)::value><<<1, 1024, 0, h->s_compute>>>(
+                pa, (int) h->total_dec, (int) h->halo_fir + 1, sp.k0, (uint32_t *) ((char *) h->scalars.p + 344));
+        });
         h->launches++;
         CU(h, cudaGetLastError());
         return OOKD_OK;
@@ -1728,9 +1771,10 @@ int ookd_gpu_decode_begin(ookd_gpu *h, const int16_t *iq, int iq_is_device_ptr, 
     constexpr u64 TILE = SCREEN_L;                             // piece boundaries: whole tiles of either kernel
     CU(h, cudaEventRecord(h->ev_f0, h->s_compute));
     if (!iq_is_device_ptr) {
-        if ((rc = ensure(h, h->in, n_have * 4 + 16))) return rc;
+        const u64 bps = h->in_bytes;
+        if ((rc = ensure(h, h->in, n_have * bps + 16))) return rc;
         d_in = (const uint32_t *) h->in.p;
-        const u64 piece = 16ull << 20;                         // 16 Mi samples = 64 MiB per copy
+        const u64 piece = 16ull << 20;                         // 16 Mi samples = 64 MiB (SC16Q11) per copy
         const u64 n_pieces = n_have ? (n_have + piece - 1) / piece : 0;
         while (h->ev_piece.size() < n_pieces) {
             cudaEvent_t e;
@@ -1740,7 +1784,7 @@ int ookd_gpu_decode_begin(ookd_gpu *h, const int16_t *iq, int iq_is_device_ptr, 
         i64 o_done = h->bit_base;
         for (u64 p = 0; p < n_pieces; p++) {
             const u64 s0 = p * piece, s1 = (s0 + piece < n_have) ? s0 + piece : n_have;
-            CU(h, cudaMemcpyAsync((uint32_t *) h->in.p + s0, (const uint32_t *) iq + s0, (s1 - s0) * 4,
+            CU(h, cudaMemcpyAsync((char *) h->in.p + s0 * bps, (const char *) iq + s0 * bps, (s1 - s0) * bps,
                                   cudaMemcpyHostToDevice, h->s_copy));
             CU(h, cudaEventRecord(h->ev_piece[p], h->s_copy));
             if (h->path != FIR_GENERIC) {
@@ -2109,7 +2153,7 @@ static int filtered_common(ookd_gpu *h, const void *in, bool in_i16, bool in_dev
     int rc;
     DevBuf tmp_in, tmp_out;
     const void *d_in = in;
-    const size_t esz = in_i16 ? 4 : 8;
+    const size_t esz = in_i16 ? h->in_bytes : 8;
     if (!in_dev) {
         if ((rc = ensure(h, tmp_in, n_samples * esz + 16))) return rc;
         if (n_samples) {

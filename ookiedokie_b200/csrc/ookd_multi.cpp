@@ -22,6 +22,7 @@ struct ookd_gpu_multi {
     std::vector<ookd_gpu *> h;
     std::vector<int32_t> dev;                // CUDA device of handle g
     uint32_t halo = 0, dec = 1, spb = 1;
+    uint32_t in_bytes = 4;                   // bytes per input sample (the handles' capture format)
     uint64_t align = 1;
     uint32_t used = 0;                       // shards of the last decode
     std::vector<ookd_msg> msgs;
@@ -85,6 +86,7 @@ int ookd_gpu_multi_create(ookd_gpu_multi **out, const struct ookd_gpu_config *cf
         m->dev.push_back(gpu_ids[g]);
     }
     m->halo = ookd_gpu_halo(m->h[0]);
+    m->in_bytes = ookd_gpu_input_bytes(m->h[0]);
     m->dec = ookd_gpu_total_decimation(m->h[0]);
     m->spb = cfg->samples_per_buffer;
     m->align = (uint64_t) m->spb / gcd64(m->spb, m->dec) * m->dec;
@@ -134,7 +136,8 @@ const int16_t *shard_ptr(const ookd_gpu_multi *m, uint32_t g)
     const uint64_t ha = m->sf[g] < m->halo ? m->sf[g] : m->halo;
     if (m->iq_mode == 1) return m->dev_ptrs[g];                         // already points at sf[g] - ha on GPU g
     const uint64_t halo_avail0 = m->first_sample < m->halo ? m->first_sample : m->halo;
-    return (const int16_t *) m->iq + 2 * ((m->sf[g] - ha) - (m->first_sample - halo_avail0));   // iq[0] = sample first_sample - halo_avail0
+    // iq[0] = sample first_sample - halo_avail0
+    return (const int16_t *) ((const char *) m->iq + m->in_bytes * ((m->sf[g] - ha) - (m->first_sample - halo_avail0)));
 }
 
 int plan(ookd_gpu_multi *m, const void *iq, int iq_mode, uint64_t first_sample, uint64_t n_samples, int last,

@@ -25,6 +25,13 @@
 //
 // Tiles the tensor copy cannot serve (capture start/end, input not 16-byte aligned) take guarded
 // scalar loads into the same registers; everything after that is identical.
+//
+// 8-bit captures (FMT_CS8 / FMT_CU8, input_fmt.cuh): the raw tile is 8 KiB, brought in as EIGHT tensor copies of 1 KiB
+// (rows of 64 samples = 128 B, box = 8 rows, 128-byte swizzle), one per warp: warp W's 512 samples land at the start of
+// the 2 KiB of the stage body that warp W's own prefix rows will cover.  Lane l owns chunks 2(l&3), 2(l&3)+1 of raw row
+// l>>2 of that block and forms its statistics straight from the bytes (screen_span_stats8); the prefix rows written in
+// place then overwrite only the warp's own raw bytes, so a __syncwarp (not a CTA barrier) separates the raw reads from
+// the prefix writes.  Shared memory, the 3-stage ring and 4 CTAs/SM stay as they are (DESIGN section 3.9).
 #pragma once
 
 #include <cuda.h>
@@ -42,6 +49,7 @@ struct ScreenTmaArgs {
 constexpr int STMA_NT = 256, STMA_SPT = 16, STMA_L = STMA_NT * STMA_SPT;   // 4096 input samples per tile
 constexpr int STMA_STAGES = 3;
 constexpr int STMA_BODY = STMA_L * 4;                           // 16 KiB per stage, 1024-byte aligned (128 B swizzle)
+constexpr int STMA8_BOX_ROWS = 8;                               // 8-bit tiles: rows (of 64 samples) per copy = one warp's span
 constexpr int STMA_HT_MAX = 5;                                  // history spans in front of a tile (2 for T=32/D=1, 5 for dec4)
 constexpr int STMA_HIST = 384;                                  // bytes of history rows per stage: rows -3..-1
 constexpr int STMA_XY_ROWS = STMA_NT + STMA_HT_MAX;
@@ -182,11 +190,61 @@ __device__ __forceinline__ void screen_span_stats_v2(const uint32_t (&w)[16], ui
     }
 }
 
+// The same statistics, in the same (SC16Q11 word) units and bit for bit the same values, straight from 16 samples of an
+// 8-bit capture (8 registers of bytes I0,Q0,I1,Q1) with dp4a instead of widening each sample first:
+//   CS8, word 16 k:             |word|^2 = 256 (kI^2 + kQ^2)              -> pre = 256 * (running sum of dp4a(x, x & half))
+//   CU8, word 16 v - 2040:      |word|^2 = (16 v - 2040)^2 = 4161600 - 256 v (255 - v) per component, 255 - v = ~v as a byte
+//                               -> pre = 8323200 n - 256 * (running sum of unsigned dp4a(x, ~x & half))
+//   sums of I (Q): 16 * (dp4a of the I (Q) bytes with ones), - 2040 per sample for CU8.
+// |word| <= 2048, so a span's total is at most 16 * 2 * 2^22 = 2^27 (and the SC16Q11 form's range guard, hi_total < 2^20,
+// always holds there as well): no guard, tot = pre[15].  Every intermediate is exact in 32 bits (CU8: the dp4a sum is at
+// most 16 * 2 * 127 * 128 < 2^20, 8323200 * 16 < 2^27).
+template <int FMT>
+__device__ __forceinline__ void screen_span_stats8(const uint32_t (&x)[8], uint32_t (&pre)[16], int &sx, int &sy,
+                                                   uint32_t &tot, uint32_t k0)
+{
+    uint32_t acc = 0;
+#pragma unroll
+    for (int j = 0; j < 8; j++) {
+#pragma unroll
+        for (int h = 0; h < 2; h++) {
+            const uint32_t half = h ? 0xFFFF0000u : 0x0000FFFFu;
+            const int e = 2 * j + h;
+            if constexpr (FMT == FMT_CU8) {
+                acc = __dp4a(x[j], ~x[j] & half, acc);                        // unsigned: v (255 - v), I and Q
+                pre[e] = 8323200u * (uint32_t) (e + 1) - 256u * acc;
+            } else {
+                acc = (uint32_t) __dp4a((int) x[j], (int) (x[j] & half), (int) acc);   // signed: k^2, I and Q
+                pre[e] = acc << 8;
+            }
+        }
+    }
+    tot = pre[15];
+    if (tot >= k0) {
+        int xs = 0, ys = 0;
+#pragma unroll
+        for (int j = 0; j < 8; j++) {
+            if constexpr (FMT == FMT_CU8) {
+                xs = (int) __dp4a(x[j], 0x00010001u, (uint32_t) xs);
+                ys = (int) __dp4a(x[j], 0x01000100u, (uint32_t) ys);
+            } else {
+                xs = __dp4a((int) x[j], 0x00010001, xs);
+                ys = __dp4a((int) x[j], 0x01000100, ys);
+            }
+        }
+        sx = (FMT == FMT_CU8) ? 16 * xs - 16 * 2040 : 16 * xs;
+        sy = (FMT == FMT_CU8) ? 16 * ys - 16 * 2040 : 16 * ys;
+    } else {
+        sx = OOKD_XY_QUIET;
+        sy = 0;
+    }
+}
+
 // ADAPT: the decode is adaptive (short captures: a probe kernel chose between this form and FMA screening; both are
 // enqueued and the one not chosen returns at once).  A separate instantiation, so that the plain form's code is untouched.
 // (__maxnreg__(64) rather than __launch_bounds__(256, 4): same occupancy, but ptxas then keeps three more values in
 // registers and the kernel measures 4 % faster)
-template <int DEC, bool ADAPT>
+template <int DEC, bool ADAPT, int FMT>
 __global__ void __maxnreg__(64)
 fir_screen_tma_kernel(const __grid_constant__ CUtensorMap tmap, const ScreenTmaArgs ta, const ScreenParams sp)
 {
@@ -194,6 +252,7 @@ fir_screen_tma_kernel(const __grid_constant__ CUtensorMap tmap, const ScreenTmaA
     constexpr int NT = STMA_NT, SPT = STMA_SPT, L = STMA_L, NS = STMA_STAGES;
     constexpr int HT = (DEC == 1) ? 2 : 5;                     // history spans
     constexpr int LOUT = L / DEC;                              // outputs per tile
+    constexpr int LOG_RS = (FMT == FMT_SC16Q11) ? 5 : 6;       // samples per 128-byte tensor row: 32 or 64
     extern __shared__ __align__(1024) uint8_t smem_raw[];
 
     const ScreenArgs &sa = ta.s;
@@ -225,17 +284,24 @@ fir_screen_tma_kernel(const __grid_constant__ CUtensorMap tmap, const ScreenTmaA
 
     auto tile_fast = [&](uint32_t tile) -> bool { return smem_aligned && tile >= ta.fast_lo && tile < ta.fast_hi; };
     auto tile_in0 = [&](uint32_t tile) -> i64 { return (a.out_lo + (i64) tile * LOUT) * DEC; };   // first input of a tile
-    auto tile_row = [&](uint32_t tile) -> int32_t { return (int32_t) ((tile_in0(tile) - ta.row0_sample) >> 5); };
+    auto tile_row = [&](uint32_t tile) -> int32_t { return (int32_t) ((tile_in0(tile) - ta.row0_sample) >> LOG_RS); };
     auto issue = [&](uint32_t tile, int s) {
         const uint32_t bar = bar0 + 8 * s;
-        mbar_expect_tx(bar, L * 4);
-        tma_load_tile(body0 + s * STMA_BODY, &tmap, tile_row(tile), bar);
+        mbar_expect_tx(bar, L * in_bytes<FMT>());
+        if constexpr (FMT == FMT_SC16Q11) {
+            tma_load_tile(body0 + s * STMA_BODY, &tmap, tile_row(tile), bar);
+        } else {
+#pragma unroll
+            for (int w = 0; w < NT / 32; w++) {                 // warp w's samples into the 2 KiB its prefix rows will use
+                tma_load_tile(body0 + s * STMA_BODY + 2048 * w, &tmap, tile_row(tile) + STMA8_BOX_ROWS * w, bar);
+            }
+        }
     };
     auto load_span_slow = [&](i64 g, uint32_t (&w)[16]) {
 #pragma unroll
         for (int e = 0; e < 16; e++) {
             const i64 ge = g + e;
-            w[e] = (ge >= 0 && ge >= a.in_base && ge < a.in_valid_end) ? __ldg(a.in + (ge - a.in_base)) : 0u;
+            w[e] = (ge >= 0 && ge >= a.in_base && ge < a.in_valid_end) ? load_word<FMT>(a.in, ge - a.in_base) : 0u;
         }
     };
     // base address of the row of virtual thread uu (>= 0: body, < 0: history rows) of stage s
@@ -279,21 +345,42 @@ fir_screen_tma_kernel(const __grid_constant__ CUtensorMap tmap, const ScreenTmaA
         const uint32_t body = body0 + s * STMA_BODY;
         const uint32_t hist = hist0 + s * STMA_HIST;
         const i64 o0 = a.out_lo + (i64) tile * LOUT;
-        uint32_t w[16];
-        if (tile_fast(tile)) {
-            mbar_wait(bar0 + 8 * s, (phases >> s) & 1u);
-            phases ^= 1u << s;
-#pragma unroll
-            for (int v = 0; v < 4; v++) {
-                const uint4 x = lds128(body + off_own[v]);
-                w[4 * v] = x.x; w[4 * v + 1] = x.y; w[4 * v + 2] = x.z; w[4 * v + 3] = x.w;
-            }
-        } else {
-            load_span_slow(tile_in0(tile) + (i64) u * SPT, w);
-        }
         uint32_t pre[SPT], tot_own;                                         // tot_own bit 31 = "span out of range"
         int sx, sy;
-        screen_span_stats_v2(w, pre, sx, sy, tot_own, sp.k0);
+        if constexpr (FMT == FMT_SC16Q11) {
+            uint32_t w[16];
+            if (tile_fast(tile)) {
+                mbar_wait(bar0 + 8 * s, (phases >> s) & 1u);
+                phases ^= 1u << s;
+#pragma unroll
+                for (int v = 0; v < 4; v++) {
+                    const uint4 x = lds128(body + off_own[v]);
+                    w[4 * v] = x.x; w[4 * v + 1] = x.y; w[4 * v + 2] = x.z; w[4 * v + 3] = x.w;
+                }
+            } else {
+                load_span_slow(tile_in0(tile) + (i64) u * SPT, w);
+            }
+            screen_span_stats_v2(w, pre, sx, sy, tot_own, sp.k0);
+        } else {
+            if (tile_fast(tile)) {
+                mbar_wait(bar0 + 8 * s, (phases >> s) & 1u);
+                phases ^= 1u << s;
+                const int r = (u & 31) >> 2;                     // raw row of 64 samples in the warp's block; chunks 2(u&3), 2(u&3)+1
+                const uint32_t blk = body + 2048 * (u >> 5);
+                uint32_t x[8];
+#pragma unroll
+                for (int v = 0; v < 2; v++) {
+                    const uint4 c = lds128(blk + r * 128 + ((((u & 3) << 1 | v) ^ r) << 4));
+                    x[4 * v] = c.x; x[4 * v + 1] = c.y; x[4 * v + 2] = c.z; x[4 * v + 3] = c.w;
+                }
+                screen_span_stats8<FMT>(x, pre, sx, sy, tot_own, sp.k0);
+            } else {
+                uint32_t w[16];
+                load_span_slow(tile_in0(tile) + (i64) u * SPT, w);
+                screen_span_stats_v2(w, pre, sx, sy, tot_own, sp.k0);
+            }
+            __syncwarp();                                        // the warp's raw bytes are read before its prefix rows overwrite them
+        }
         {
             uint32_t p[16];
 #pragma unroll

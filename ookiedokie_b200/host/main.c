@@ -2,7 +2,8 @@
  * ookiedokie-b200 -- command line front end with the reference's option surface
  * (reference src/main.c:90-181) driving the B200 receive path.
  *
- * Supported SDR type: bladerf_file (SC16Q11 capture files).  Options that only configure live
+ * Supported SDR types: bladerf_file (SC16Q11 capture files), and for --rx also cu8_file (RTL-SDR, uint8 I,Q) and
+ * cs8_file (HackRF / bladeRF SC8_Q7, int8 I,Q), decoded natively on the GPU.  Options that only configure live
  * bladeRF hardware (frequency, bandwidth, gain, stream sizing) are accepted and ignored.
  */
 #include <getopt.h>
@@ -63,9 +64,10 @@ static const struct option long_options[] = {
 static void usage(const char *argv0)
 {
     printf("ookiedokie-b200: receive OOK modulated signals on a B200 GPU\n\n");
-    printf("Usage: %s <--rx | --tx> bladerf_file [options]\n\n", argv0);
+    printf("Usage: %s <--rx | --tx> bladerf_file [options]\n", argv0);
+    printf("       %s --rx <cu8_file | cs8_file> [options]\n\n", argv0);
     printf("Required parameters:\n");
-    printf("  -r, --rx <SDR type>           Receive data (SDR type: bladerf_file).\n");
+    printf("  -r, --rx <SDR type>           Receive data (SDR type: bladerf_file, cu8_file, cs8_file).\n");
     printf("  -t, --tx <SDR type>           Generate a capture (SDR type: bladerf_file).\n");
     printf("  -d, --device <str>            Target OOK device name.\n\n");
     printf("Transmit options:\n");
@@ -80,7 +82,8 @@ static void usage(const char *argv0)
     printf("  -B, --rx-rec-dig <filename>   Save the digital signal transitions to a CSV file.\n");
     printf("  --rx-fmt <fmt>                \"csv\" or \"pretty\" (default).\n\n");
     printf("SDR configuration options:\n");
-    printf("  -A, --sdr-args <file>         SC16Q11 capture file.\n");
+    printf("  -A, --sdr-args <file>         Capture file (\"-\": stdin): SC16Q11 for bladerf_file, interleaved\n");
+    printf("                                uint8 I,Q for cu8_file, int8 I,Q for cs8_file.\n");
     printf("  -s, --samplerate <rate>       Sample rate of the capture (K/M/G suffixes allowed).\n\n");
     printf("Sample stream options:\n");
     printf("  --samples-per-buffer <n>      Buffer size the decode semantics are defined on.\n\n");
@@ -146,9 +149,19 @@ int main(int argc, char *argv[])
                     fprintf(stderr, "Error: --rx or --tx already specified.\n");
                     return EXIT_FAILURE;
                 }
-                if (strcasecmp(optarg, "bladerf_file")) {
-                    fprintf(stderr, "Error: SDR type \"%s\" is not available; this build supports bladerf_file.\n",
+                if (!strcasecmp(optarg, "bladerf_file")) {
+                    cfg.input_flags = 0;
+                } else if (c == 'r' && !strcasecmp(optarg, "cu8_file")) {
+                    cfg.input_flags = OOKD_FLAG_INPUT_CU8;
+                } else if (c == 'r' && !strcasecmp(optarg, "cs8_file")) {
+                    cfg.input_flags = OOKD_FLAG_INPUT_CS8;
+                } else if (c == 't' && (!strcasecmp(optarg, "cu8_file") || !strcasecmp(optarg, "cs8_file"))) {
+                    fprintf(stderr, "Error: --tx writes SC16Q11 captures only (bladerf_file); \"%s\" is a receive type.\n",
                             optarg);
+                    return EXIT_FAILURE;
+                } else {
+                    fprintf(stderr, "Error: SDR type \"%s\" is not available; this build supports bladerf_file, "
+                            "and cu8_file and cs8_file for --rx.\n", optarg);
                     return EXIT_FAILURE;
                 }
                 direction = (c == 't');

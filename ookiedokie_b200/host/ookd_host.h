@@ -116,6 +116,8 @@ struct ookd_cfg {                       /* the fields of struct ookiedokie_cfg t
     const struct ookd_keyval_list *device_params;
     int      gpu_id;                    /* CUDA ordinal, -1 => current                        */
     FILE    *out;                       /* message output, NULL => stdout                     */
+    uint32_t input_flags;               /* capture format: 0 SC16Q11 (bladerf_file), OOKD_FLAG_INPUT_CS8 (cs8_file) or
+                                           OOKD_FLAG_INPUT_CU8 (cu8_file); recordings stay SC16Q11  */
 };
 void ookd_cfg_init(struct ookd_cfg *cfg);               /* defaults of src/ookiedokie_cfg.c:27-38 */
 int  ookd_rx(const struct ookd_cfg *cfg);               /* 0 on success */

@@ -92,13 +92,14 @@ static void init_signal_handling(void)
 void ookd_rx_request_stop(void) { g_running = 0; }
 
 /* ---- capture reader: a thread that keeps a ring of pinned window buffers filled while the GPU decodes ----
- * Slot layout: [halo samples of history][window samples].  The reader copies the tail of the previous window in front
+ * Slot layout: [halo samples of history][window samples], in the capture's format (bps bytes per sample: 4 SC16Q11,
+ * 2 CU8 / CS8; a trailing partial sample is ignored).  The reader copies the tail of the previous window in front
  * of the next one itself, so a slot is self-contained when it is handed over (sdr_bladerf_file_rx's role,
  * src/sdr/bladeRF_file.c:97-126; the zero padding of the last buffer happens inside the decode). */
 #define RX_SLOTS 3
 
 struct rx_slot {
-    int16_t *buf;               /* pinned, (halo + window) samples                                  */
+    uint8_t *buf;               /* pinned, (halo + window) samples                                  */
     size_t have;                /* samples read into the window part                                */
     uint64_t first_sample;
     bool last;                  /* nothing follows this window (EOF, read error or stop request)    */
@@ -109,6 +110,7 @@ struct rx_reader {
     FILE *in;
     struct rx_slot slot[RX_SLOTS];
     uint64_t window, halo;
+    size_t bps;                 /* bytes per sample */
     pthread_t thread;
     pthread_mutex_t mu;
     pthread_cond_t cv;
@@ -128,11 +130,11 @@ static void *reader_main(void *arg)
         pthread_mutex_unlock(&r->mu);
         if (w > 0) {                                        /* history: the tail of the previous window */
             const struct rx_slot *p = &r->slot[(w - 1) % RX_SLOTS];
-            memcpy(s->buf, p->buf + 2 * (size_t) p->have, (size_t) r->halo * 4);      /* [have, have + halo) of p */
+            memcpy(s->buf, p->buf + r->bps * (size_t) p->have, (size_t) r->halo * r->bps);      /* [have, have + halo) of p */
         }
         size_t have = 0;
         if (g_running) {
-            have = fread(s->buf + 2 * (size_t) r->halo, 4, (size_t) r->window, r->in);
+            have = fread(s->buf + r->bps * (size_t) r->halo, r->bps, (size_t) r->window, r->in);
         }
         bool last = (have < r->window) || !g_running;
         if (!last) {                                        /* exactly full: is anything left? */
@@ -246,12 +248,38 @@ static int write_rec_filtered(struct rx_out *o, ookd_gpu *gpu)
 }
 
 /* --rx-rec-input (src/ookiedokie.c:248-253): the raw buffers, the last one zero padded like sdr_bladerf_file_rx
- * leaves it (int16 -> float -> (int16_t)(x * 2048.0f) is the identity) */
-static int write_rec_input(struct rx_out *o, const struct rx_slot *s, uint64_t halo, uint64_t spb)
+ * leaves it (int16 -> float -> (int16_t)(x * 2048.0f) is the identity).  The recording is an SC16Q11 file whatever the
+ * capture's format: 8-bit samples are written widened (CS8 k -> 16 k, CU8 v -> 16 v - 2040, the value they stand
+ * for), and the padding is SC16Q11 zeros. */
+static int write_rec_input(struct rx_out *o, const struct rx_slot *s, uint64_t halo, uint64_t spb, uint32_t input_flags)
 {
-    if (fwrite(s->buf + 2 * (size_t) halo, 4, s->have, o->rec) != s->have) {
-        log_error("Sample file write was truncated.\n");
-        return OOKD_ERR_STATE;
+    if (!input_flags) {
+        if (fwrite(s->buf + 4 * (size_t) halo, 4, s->have, o->rec) != s->have) {
+            log_error("Sample file write was truncated.\n");
+            return OOKD_ERR_STATE;
+        }
+    } else {
+        const uint8_t *src = s->buf + 2 * (size_t) halo;
+        const size_t step = 1u << 16;
+        if (o->rec_cap < step) {
+            free(o->rec_buf);
+            o->rec_buf = malloc(step * 4);
+            o->rec_cap = o->rec_buf ? step : 0;
+            if (!o->rec_buf) {
+                return OOKD_ERR_NOMEM;
+            }
+        }
+        for (size_t i0 = 0; i0 < s->have; i0 += step) {
+            const size_t n = s->have - i0 < step ? s->have - i0 : step;
+            for (size_t k = 0; k < 2 * n; k++) {
+                const uint8_t b = src[2 * i0 + k];
+                o->rec_buf[k] = (input_flags & OOKD_FLAG_INPUT_CS8) ? (int16_t) (16 * (int8_t) b) : (int16_t) (16 * b - 2040);
+            }
+            if (fwrite(o->rec_buf, 4, n, o->rec) != n) {
+                log_error("Sample file write was truncated.\n");
+                return OOKD_ERR_STATE;
+            }
+        }
     }
     if (s->last && (s->have % spb)) {
         const size_t pad = (size_t) (spb - s->have % spb);
@@ -337,6 +365,7 @@ int ookd_rx(const struct ookd_cfg *cfg)
     gc.threshold = cfg->rx_threshold;
     gc.samples_per_buffer = cfg->samples_per_buffer;
     gc.device_id = cfg->gpu_id;
+    gc.flags = cfg->input_flags;
     const unsigned n_gpus = cfg->n_gpus > 1 ? cfg->n_gpus : 1;
     int rc;
     uint32_t halo;
@@ -387,15 +416,16 @@ int ookd_rx(const struct ookd_cfg *cfg)
     }
     rd.window = window;
     rd.halo = halo;
+    rd.bps = cfg->input_flags ? 2 : 4;
     pthread_mutex_init(&rd.mu, NULL);
     pthread_cond_init(&rd.cv, NULL);
     for (int i = 0; i < RX_SLOTS; i++) {
-        rd.slot[i].buf = ookd_gpu_host_alloc(((size_t) window + halo) * 4);
+        rd.slot[i].buf = ookd_gpu_host_alloc(((size_t) window + halo) * rd.bps);
         if (!rd.slot[i].buf) {
             log_error("Failed to allocate the pinned staging buffers.\n");
             goto out;
         }
-        memset(rd.slot[i].buf, 0, (size_t) halo * 4);
+        memset(rd.slot[i].buf, 0, (size_t) halo * rd.bps);
     }
     g_running = 1;
     init_signal_handling();
@@ -413,7 +443,7 @@ int ookd_rx(const struct ookd_cfg *cfg)
         struct ookd_gpu_result res;
         struct ookd_sm_carry exit_carry;
         const uint64_t halo_avail = cur->first_sample < halo ? cur->first_sample : halo;
-        const int16_t *p = cur->buf + 2 * ((size_t) halo - halo_avail);
+        const int16_t *p = (const int16_t *) (cur->buf + rd.bps * ((size_t) halo - halo_avail));
         if (cur->have == 0) {                               /* zero-length read: EOF, iteration discarded (ookiedokie.c:243-246) */
             reader_release(&rd, w);
             break;
@@ -442,7 +472,7 @@ int ookd_rx(const struct ookd_cfg *cfg)
                 next = reader_wait(&rd, w + 1);
                 if (next->have > 0) {
                     const uint64_t ha = next->first_sample < halo ? next->first_sample : halo;
-                    rc = ookd_gpu_decode_begin(gpu[(w + 1) % 2], next->buf + 2 * ((size_t) halo - ha), 0, next->first_sample,
+                    rc = ookd_gpu_decode_begin(gpu[(w + 1) % 2], (const int16_t *) (next->buf + rd.bps * ((size_t) halo - ha)), 0, next->first_sample,
                                                next->have, next->last, NULL);
                     if (rc != OOKD_OK) {
                         log_error("GPU decode failed: %s (%s)\n", ookd_gpu_strerror(rc), ookd_gpu_last_error(gpu[(w + 1) % 2]));
@@ -469,7 +499,7 @@ int ookd_rx(const struct ookd_cfg *cfg)
 
         if (o.rec) {
             if (rec_input) {
-                rc = write_rec_input(&o, cur, halo, spb);
+                rc = write_rec_input(&o, cur, halo, spb, cfg->input_flags);
             } else if (multi) {
                 rc = OOKD_OK;
                 for (uint32_t q = 0; rc == OOKD_OK && q < ookd_gpu_multi_shards_used(multi); q++) {
