@@ -120,7 +120,8 @@ int  ookd_sm_compile(const struct ookd_sm_desc *desc, struct ookd_sm_compiled *o
 void ookd_sm_compiled_free(struct ookd_sm_compiled *c);
 
 /* Smallest float p with sqrtf(p) >= thr, so that (re*re+im*im >= p) is the
- * reference's (sqrtf(re*re+im*im) >= thr), src/ookiedokie.c:177. */
+ * reference's (sqrtf(re*re+im*im) >= thr), src/ookiedokie.c:177.  A NaN
+ * threshold gives NaN (the reference decides 0 for every power). */
 float ookd_power_threshold(float thr);
 
 /* ---- results ---- */

@@ -631,14 +631,21 @@ int run_generic_chain(ookd_gpu *h, const void *d_in, bool in_is_i16, i64 in_base
 
 // complexf_to_sc16q11 (src/complexf.h:87-96): (int16_t) (x * 2048.0f), i.e. rounded multiply, truncation towards
 // zero, low 16 bits -- what the reference's post-filter recorder writes (sdr_bladerf_file_tx).
+// The float-to-int32 conversion is x86's cvttss2si: NaN and |v| >= 2^31 (infinities included) give INT_MIN, where
+// __float2int_rz would saturate.
+__device__ __forceinline__ uint32_t recorder_word(float x)
+{
+    const float v = __fmul_rn(x, 2048.0f);
+    const int i = fabsf(v) < 2147483648.0f ? __float2int_rz(v) : INT_MIN;
+    return (uint32_t) (uint16_t) (int16_t) i;
+}
+
 __global__ void __launch_bounds__(256) cf_to_sc16q11_kernel(const float2 *in, uint32_t *out, u64 n)
 {
     const u64 i = (u64) blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const float2 v = in[i];
-    const uint32_t re = (uint32_t) (uint16_t) (int16_t) __float2int_rz(__fmul_rn(v.x, 2048.0f));
-    const uint32_t im = (uint32_t) (uint16_t) (int16_t) __float2int_rz(__fmul_rn(v.y, 2048.0f));
-    out[i] = re | (im << 16);
+    out[i] = recorder_word(v.x) | (recorder_word(v.y) << 16);
 }
 
 // ---- state machine stage + message gather; fills res ----
@@ -1593,11 +1600,21 @@ int ookd_gpu_create(ookd_gpu **out, const struct ookd_gpu_config *cfg)
             h->path = FIR_TILED_1STAGE_32;
         }
     }
-    const bool pstar_ok = h->pstar > 0.0f && h->pstar < 3.0e38f;
+    // The screens' proofs hold where the reference's arithmetic has relative rounding errors only (DESIGN §3.1): a
+    // finite P* of at least 2^-100 (below, its power is rounded on the subnormal grid in absolute steps of 2^-149;
+    // thr <= 0 gives P* = 0 and NaN gives NaN), and taps for which no partial sum can overflow (an infinite sum makes
+    // NaN from inf - inf).  Elsewhere the exact kernels decide.
+    double in_max = 16.0;                                   // |I|, |Q| <= 32768 / 2048
+    for (const Stage &st : h->stages) {
+        double l1 = 0.0;
+        for (float t : st.taps) l1 += fabs((double) t);
+        in_max *= l1;
+    }
+    const bool in_domain = h->pstar >= 0x1p-100f && h->pstar < 3.0e38f && in_max < 0x1p126;
     if (!(h->flags & OOKD_FLAG_FORCE_GENERIC) && h->stages.size() == 2 &&
         h->stages[0].T == 16 && h->stages[0].D == 2 && h->stages[1].T == 32 && h->stages[1].D == 2) {
         h->path = FIR_SCREEN_DEC4;
-        h->screen2 = !(h->flags & OOKD_FLAG_NO_SCREEN) && pstar_ok;
+        h->screen2 = !(h->flags & OOKD_FLAG_NO_SCREEN) && in_domain;
     }
     h->n_sm = (unsigned) prop.multiProcessorCount;
     {
@@ -1611,11 +1628,8 @@ int ookd_gpu_create(ookd_gpu **out, const struct ookd_gpu_config *cfg)
             }
         }
     }
-    // the screen needs a finite positive power threshold (thr <= 0 decides 1 everywhere, NaN 0 everywhere;
-    // the exact kernels handle those directly)
-    h->screen = (h->path == FIR_TILED_1STAGE_32) && !(h->flags & OOKD_FLAG_NO_SCREEN) && h->pstar > 0.0f &&
-                h->pstar < 3.0e38f;
-    h->fma_ok = (h->path == FIR_TILED_1STAGE_32 || h->path == FIR_SCREEN_DEC4) && !(h->flags & OOKD_FLAG_NO_SCREEN) && pstar_ok;
+    h->screen = (h->path == FIR_TILED_1STAGE_32) && !(h->flags & OOKD_FLAG_NO_SCREEN) && in_domain;
+    h->fma_ok = (h->path == FIR_TILED_1STAGE_32 || h->path == FIR_SCREEN_DEC4) && !(h->flags & OOKD_FLAG_NO_SCREEN) && in_domain;
     if (h->fma_ok && (h->flags & OOKD_FLAG_FMA_SCREEN)) {               // start in FMA screening straight away
         h->screen = false;
         h->screen2 = false;

@@ -230,13 +230,13 @@ void ookd_sm_compiled_free(struct ookd_sm_compiled *c)
  * of powers that pass is an up-set {p >= P*}; P* is found by walking the few
  * floats around thr*thr.  (thr*thr itself is wrong by one ulp for the default
  * thr = 0.1f.)  thr <= 0 passes every power (P* = 0); a NaN threshold passes
- * nothing (+inf is returned and no finite power reaches it; inf >= inf would,
- * but a power of inf cannot be produced from int16 inputs and finite taps).
+ * nothing, not even a power that overflowed to +inf, so NaN is returned: every
+ * comparison with it is false.
  */
 float ookd_power_threshold(float thr)
 {
     if (isnan(thr)) {
-        return INFINITY;
+        return thr;
     }
     if (thr <= 0.0f) {
         return 0.0f;

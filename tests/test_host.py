@@ -157,7 +157,11 @@ def test_sm_compile_rejects_bad_descriptors():
         B.sm_compile(bad, 36, 3000000)
 
 
-@pytest.mark.parametrize("thr", [0.1, 0.0, 1.0, 0.5, 0.25, 0.3, 1e-3, 0.0999, 0.7071, 3.1e-5])
+@pytest.mark.parametrize("thr", [0.1, 0.0, 1.0, 0.5, 0.25, 0.3, 1e-3, 0.0999, 0.7071, 3.1e-5,
+                                 # P* subnormal, squares that underflow, subnormal thresholds
+                                 2.0 ** -70, 1e-20, 3e-22, 1e-30, 1e-40, 2.0 ** -149,
+                                 # squares that overflow, and inf
+                                 1e19, 1.8446742e19, 2e19, 3e38, float("inf")])
 def test_power_threshold_is_the_exact_sqrt_boundary(thr):
     t = np.float32(thr)
     p = np.float32(B.power_threshold(thr))
@@ -167,6 +171,13 @@ def test_power_threshold_is_the_exact_sqrt_boundary(thr):
     assert np.sqrt(p, dtype=np.float32) >= t
     below = np.nextafter(p, np.float32(0), dtype=np.float32)
     assert np.sqrt(below, dtype=np.float32) < t
+
+
+def test_power_threshold_of_nan_is_nan():
+    # the reference's sqrtf(p) >= NaN is false for every power, +inf included
+    assert np.isnan(B.power_threshold(float("nan")))
+    assert B.power_threshold(float("inf")) == float("inf")
+    assert B.power_threshold(2.0 ** -70) == 2.0 ** -140
 
 
 def test_power_threshold_default_is_not_thr_squared():
@@ -218,6 +229,20 @@ def test_formatter_known_rows():
     assert rem.format(d3)[-1] == ("Button", "0x1234")
     neg = nexa.message({"Temperature (C)": "-12.3"})
     assert dict(nexa.format(neg))["Temperature (C)"] == "-12.300"
+
+
+def test_filter_loader_matches_oracle_loader_on_extreme_taps(tmp_path):
+    """Exponent notation, subnormal and huge taps, signed zeros: the C loader rounds every number as the oracle does."""
+    taps = ["1e-3", "-2.5E+2", "1E0", "0.5e1", "1e-40", "-1.4e-45", "3e-39", "1.1754942e-38", "1e30", "-3.4e38",
+            "3.4028235e38", "0.0", "-0.0", "0.1", "123456789", "7e-46", "1.0000000596046448"]
+    p = tmp_path / "extreme.json"
+    p.write_text('{"filter": {"stages": [{"decimation": 3, "taps": [%s]}, {"taps": [%s]}]}}'
+                 % (", ".join(taps), ", ".join(reversed(taps))))
+    mine, ref = H.Fir(str(p)).stages, O.load_filter(str(p))
+    assert len(mine) == len(ref) == 2
+    for (d0, t0), (d1, t1) in zip(mine, ref):
+        assert d0 == d1 and np.array_equal(t0.view(np.uint32), t1.view(np.uint32))
+    assert ref[0][1].view(np.uint32)[12] == 0x80000000 and 0 < abs(ref[0][1][4]) < np.finfo(np.float32).tiny
 
 
 def test_json_reader_rejects_duplicates_and_garbage(tmp_path):
