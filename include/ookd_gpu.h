@@ -124,6 +124,43 @@ void ookd_sm_compiled_free(struct ookd_sm_compiled *c);
  * threshold gives NaN (the reference decides 0 for every power). */
 float ookd_power_threshold(float thr);
 
+/* ---- Tuning: decode a transmitter that sits off the capture's centre frequency ----
+ * With ookd_gpu_config.tune_step = step != 0, every entry point that reads a capture decodes T(x) instead of x:
+ * ookd_gpu_decode, _decode_shard, _decode_begin / _end, _resolve, ookd_gpu_batch_decode (each handle with its own
+ * step), the ookd_gpu_multi_* calls, sub-windows, ookd_gpu_filtered and ookd_gpu_filtered_sc16q11.
+ * ookd_gpu_filter_cf takes float samples, not a capture, and is unaffected.  T(x) is an SC16Q11 capture defined by
+ * integer arithmetic alone, so a tuned decode of x equals, bit for bit, the untuned decode of T(x):
+ *
+ *   Phase step.  step is a uint32, the phase advance per input sample in units of 2^-32 turns.
+ *     ookd_tune_step(offset_hz, samplerate, &step) computes llround(offset_hz / samplerate * 2^32) modulo 2^32, so
+ *     negative offsets wrap to two's complement.  It returns OOKD_ERR_ARG if offset_hz is not finite, samplerate is
+ *     0, or |offset_hz| >= samplerate / 2.  offset_hz is where the transmitter sits in the capture: +250 kHz means
+ *     250 kHz above centre.
+ *   Phase of sample n.  n is the global index in the capture (sample 0 is the first sample of the file).
+ *     phi(n) = (uint32)(n * step), the low 32 bits of the product, with no running accumulator, so shards,
+ *     sub-windows, windows of the CLI and multi-GPU splits all see the same phase.  Table index k = phi(n) >> 22.
+ *   Table.  S[j] = round(32767 * sin(2*pi*j/1024)) for j = 0..256, ties away from zero (ookd_tune_quarter).
+ *     With q = k >> 8 and r = k & 255:
+ *       q = 0: (c, s) = ( S[256-r],  S[r])
+ *       q = 1: (c, s) = (-S[r],      S[256-r])
+ *       q = 2: (c, s) = (-S[256-r], -S[r])
+ *       q = 3: (c, s) = ( S[r],     -S[256-r])
+ *   Rotation by e^{-j phi}, in int32 with >> an arithmetic shift:
+ *       I' = sat16((I*c + Q*s + 16384) >> 15)
+ *       Q' = sat16((Q*c - I*s + 16384) >> 15)
+ *     sat16 clamps to [-32768, 32767].  With |I|, |Q| <= 32768 and |c|, |s| <= 32767 every intermediate stays below
+ *     2^31; the clamp is reachable only by full-scale SC16Q11 input.
+ *   Order with the 8-bit formats.  An 8-bit sample is widened to its word first (CS8 16k, CU8 16v - 2040), then
+ *     rotated.
+ *   Outside the capture.  The history before sample 0 and the EOF padding stay word 0 (the rotation of 0 is 0).
+ *   Off.  step == 0 means no tuning, and the handle runs exactly the untuned kernels.
+ * T is a 12-bit-accurate NCO: spurs about 60 dB down and a gain of 32767/32768. */
+extern const int16_t ookd_tune_quarter[257];
+int ookd_tune_step(double offset_hz, uint32_t samplerate, uint32_t *step);
+/* CPU form of T: n_samples SC16Q11 samples (interleaved int16 I,Q) whose first one is global sample first_sample;
+ * out may equal in.  8-bit captures are widened to SC16Q11 words first. */
+int ookd_tune_sc16q11(const int16_t *in, int16_t *out, uint64_t first_sample, uint64_t n_samples, uint32_t step);
+
 /* ---- results ---- */
 struct ookd_msg {
     uint64_t out_sample;                     /* post-decimation index of the sample that
@@ -172,6 +209,8 @@ struct ookd_gpu_config {
                                                 (refine, edges, state machine) runs while sub-window j+1 streams.  Results
                                                 are identical; ookd_gpu_bits / ookd_gpu_filtered_sc16q11 are not available
                                                 after a decode that was cut (OOKD_ERR_STATE).  Implies sm_warmup.  0, 1: off */
+    uint32_t tune_step;                      /* != 0: decode the capture shifted down by a frequency offset (see
+                                                "Tuning" below; ookd_tune_step converts Hz).  0: off, today's kernels */
 };
 
 #define OOKD_FLAG_FORCE_GENERIC  1u          /* always use the shape-agnostic FIR kernels       */

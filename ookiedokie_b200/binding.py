@@ -36,6 +36,7 @@ INPUT_FORMATS = {"sc16q11": (0, np.int16), "cs8": (FLAG_INPUT_CS8, np.int8), "cu
 # every symbol include/ookd_gpu.h declares
 EXPORTS = [
     "ookd_sm_compile", "ookd_sm_compiled_free", "ookd_sm_idle_carry", "ookd_power_threshold",
+    "ookd_tune_step", "ookd_tune_sc16q11",
     "ookd_gpu_device_count", "ookd_gpu_strerror", "ookd_gpu_last_error",
     "ookd_gpu_create", "ookd_gpu_destroy", "ookd_gpu_decode", "ookd_gpu_decode_shard",
     "ookd_gpu_decode_begin", "ookd_gpu_decode_end", "ookd_gpu_batch_decode",
@@ -128,7 +129,7 @@ class GpuConfig(C.Structure):
     _fields_ = [("filter", C.POINTER(FilterDesc)), ("sm", C.POINTER(SmDesc)), ("threshold", C.c_float),
                 ("samples_per_buffer", C.c_uint32), ("device_id", C.c_int32), ("flags", C.c_uint32),
                 ("sm_chunk_buffers", C.c_uint32), ("sm_warmup", C.c_uint32), ("sm_burst_rounds", C.c_uint32),
-                ("sub_windows", C.c_uint32)]
+                ("sub_windows", C.c_uint32), ("tune_step", C.c_uint32)]
 
 
 class GpuResult(C.Structure):
@@ -164,6 +165,10 @@ def lib():
         L.ookd_sm_idle_carry.argtypes = [C.POINTER(SmCompiled), C.POINTER(SmCarry)]
         L.ookd_power_threshold.restype = C.c_float
         L.ookd_power_threshold.argtypes = [C.c_float]
+        L.ookd_tune_step.restype = C.c_int
+        L.ookd_tune_step.argtypes = [C.c_double, C.c_uint32, C.POINTER(C.c_uint32)]
+        L.ookd_tune_sc16q11.restype = C.c_int
+        L.ookd_tune_sc16q11.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32]
         L.ookd_gpu_device_count.restype = C.c_int
         L.ookd_gpu_strerror.restype = C.c_char_p
         L.ookd_gpu_strerror.argtypes = [C.c_int]
@@ -328,6 +333,31 @@ def power_threshold(thr):
     return float(lib().ookd_power_threshold(C.c_float(thr)))
 
 
+def tune_step(offset_hz, samplerate):
+    """Phase step of a transmitter offset_hz from the capture's centre at samplerate samples/s (ookd_tune_step):
+    llround(offset_hz / samplerate * 2^32) modulo 2^32.  ValueError if offset_hz is not finite, samplerate is 0 or
+    |offset_hz| >= samplerate / 2."""
+    if not 0 <= int(samplerate) < 2**32:
+        raise ValueError(f"samplerate {samplerate} is not a uint32")
+    step = C.c_uint32()
+    if lib().ookd_tune_step(C.c_double(float(offset_hz)), C.c_uint32(int(samplerate)), C.byref(step)) != 0:
+        raise ValueError(f"no tune step for an offset of {offset_hz} Hz at {samplerate} samples/s: the offset must be "
+                         f"finite and below half the sample rate in magnitude")
+    return int(step.value)
+
+
+def tune_sc16q11(iq, first_sample, step):
+    """CPU form of the tuning rotation T (ookd_tune_sc16q11): int16 I,Q samples whose first one is global sample
+    first_sample -> the rotated samples, same shape."""
+    a = np.ascontiguousarray(iq, dtype=np.int16)
+    out = np.empty_like(a)
+    rc = lib().ookd_tune_sc16q11(C.c_void_p(a.ctypes.data), C.c_void_p(out.ctypes.data), C.c_uint64(int(first_sample)),
+                                 C.c_uint64(a.size // 2), C.c_uint32(int(step)))
+    if rc != 0:
+        raise OokdError(f"ookd_tune_sc16q11: {lib().ookd_gpu_strerror(rc).decode()}")
+    return out
+
+
 def device_count():
     return int(lib().ookd_gpu_device_count())
 
@@ -366,10 +396,13 @@ def _as_ptr(iq, input_format="sc16q11"):
 
 class Gpu:
     """One ookd_gpu handle.  input_format: "sc16q11" (int16 I,Q), "cs8" (int8 I,Q) or "cu8" (uint8 I,Q) host arrays;
-    an 8-bit capture decodes exactly as its widened SC16Q11 capture does (include/ookd_gpu.h, OOKD_FLAG_INPUT_*)."""
+    an 8-bit capture decodes exactly as its widened SC16Q11 capture does (include/ookd_gpu.h, OOKD_FLAG_INPUT_*).
+    tune_step != 0 (see tune_step()): decode the capture shifted down by that frequency offset, exactly as the untuned
+    handle decodes the rotated capture T(x) (include/ookd_gpu.h, "Tuning")."""
 
     def __init__(self, filter_stages=None, sm=None, threshold=0.1, samples_per_buffer=8192, device_id=-1,
-                 flags=0, sm_chunk_buffers=0, sm_warmup=0, sm_burst_rounds=0, sub_windows=0, input_format="sc16q11"):
+                 flags=0, sm_chunk_buffers=0, sm_warmup=0, sm_burst_rounds=0, sub_windows=0, input_format="sc16q11",
+                 tune_step=0):
         flags |= _input_format(input_format, flags)[0]
         self.input_format = input_format
         L = lib()
@@ -394,6 +427,7 @@ class Gpu:
         cfg.sm_warmup = sm_warmup
         cfg.sm_burst_rounds = sm_burst_rounds
         cfg.sub_windows = sub_windows
+        cfg.tune_step = tune_step
         self.h = C.c_void_p()
         rc = L.ookd_gpu_create(C.byref(self.h), C.byref(cfg))
         if rc != 0:
@@ -535,7 +569,7 @@ class MultiGpu:
     """One ookd_gpu_multi handle: a window time-sharded over several GPUs of this process."""
 
     def __init__(self, gpu_ids, filter_stages=None, sm=None, threshold=0.1, samples_per_buffer=8192, flags=0,
-                 sm_chunk_buffers=0, input_format="sc16q11"):
+                 sm_chunk_buffers=0, input_format="sc16q11", tune_step=0):
         flags |= _input_format(input_format, flags)[0]
         self.input_format = input_format
         L = lib()
@@ -556,6 +590,7 @@ class MultiGpu:
         cfg.samples_per_buffer = samples_per_buffer
         cfg.flags = flags
         cfg.sm_chunk_buffers = sm_chunk_buffers
+        cfg.tune_step = tune_step
         ids = (C.c_int32 * len(gpu_ids))(*gpu_ids)
         self.h = C.c_void_p()
         rc = L.ookd_gpu_multi_create(C.byref(self.h), C.byref(cfg), ids, len(gpu_ids))

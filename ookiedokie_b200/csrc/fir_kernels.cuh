@@ -39,7 +39,7 @@ struct GenericStageArgs {
 };
 
 template <bool IN_I16, int FMT>
-__global__ void __launch_bounds__(256) fir_stage_generic_kernel(const GenericStageArgs a)
+__global__ void __launch_bounds__(256) fir_stage_generic_kernel(const GenericStageArgs a, const uint32_t tune_step)
 {
     extern __shared__ float s_taps[];
     for (uint32_t i = threadIdx.x; i < a.T; i += blockDim.x) {
@@ -60,7 +60,7 @@ __global__ void __launch_bounds__(256) fir_stage_generic_kernel(const GenericSta
                     if constexpr (FMT == FMT_SC16Q11) {     // (a plain load, not __ldg: its SASS is kept as it was)
                         x = sc16q11_to_float2(((const uint32_t *) a.in)[g - a.in_base]);
                     } else {
-                        x = sc16q11_to_float2(load_word<FMT>((const uint32_t *) a.in, g - a.in_base));
+                        x = sc16q11_to_float2(load_word<FMT>((const uint32_t *) a.in, g - a.in_base, g, tune_step));
                     }
                 } else {
                     x = ((const float2 *) a.in)[g - a.in_base];
@@ -143,7 +143,8 @@ struct ScreenArgs {
 // almost nothing and every group would go to the exact kernel.  256 windows spread over the capture are enough to tell:
 // fewer than 40 % provably off => FMA screening.  One small CTA, no host round trip (the FIR kernels read the verdict).
 template <int FMT>
-__global__ void __launch_bounds__(1024) screen_probe_kernel(const TiledArgs a, int dec, int window, uint32_t k0, uint32_t *mode)
+__global__ void __launch_bounds__(1024) screen_probe_kernel(const TiledArgs a, int dec, int window, uint32_t k0, uint32_t *mode,
+                                                               const uint32_t tune_step)
 {
     // 32 warps x 8 windows; lane i of a warp reads samples i, i + 32, ... of the window (coalesced)
     __shared__ uint32_t s_cnt[32];
@@ -157,7 +158,7 @@ __global__ void __launch_bounds__(1024) screen_probe_kernel(const TiledArgs a, i
         unsigned long long e = 0;
         for (int i = (int) lane; i < window; i += 32) {
             const i64 g = newest - i;
-            const uint32_t w = (g >= 0 && g >= a.in_base && g < a.in_valid_end) ? load_word<FMT>(a.in, g - a.in_base) : 0u;
+            const uint32_t w = (g >= 0 && g >= a.in_base && g < a.in_valid_end) ? load_word<FMT>(a.in, g - a.in_base, g, tune_step) : 0u;
             const long long I = (short) (w & 0xFFFFu), Q = ((int) w) >> 16;
             e += (unsigned long long) (I * I + Q * Q);
         }
@@ -215,7 +216,7 @@ __device__ __forceinline__ uint32_t fma_classify(float re, float im, float hi2, 
 
 template <int T, int R, bool FMA, bool ADAPT, int FMT>
 __global__ void __launch_bounds__(256, 2)
-fir1_tiled_kernel(const ScreenArgs sa, const TapsParam<T> taps, const FmaBand band)
+fir1_tiled_kernel(const ScreenArgs sa, const TapsParam<T> taps, const FmaBand band, const uint32_t tune_step)
 {
     constexpr int NT = 256;
     constexpr int L = NT * R;                 // outputs per tile
@@ -253,12 +254,12 @@ fir1_tiled_kernel(const ScreenArgs sa, const TapsParam<T> taps, const FmaBand ba
             const i64 g = g0 + VS * q;
             uint32_t w[VS];
             if (aligned && g >= a.in_base && g >= 0 && g + VS <= a.in_valid_end) {
-                load_words16<FMT>(a.in, g - a.in_base, w);
+                load_words16<FMT>(a.in, g - a.in_base, g, tune_step, w);
             } else {
 #pragma unroll
                 for (int e = 0; e < VS; e++) {
                     const i64 ge = g + e;
-                    w[e] = (ge >= 0 && ge >= a.in_base && ge < a.in_valid_end) ? load_word<FMT>(a.in, ge - a.in_base) : 0u;
+                    w[e] = (ge >= 0 && ge >= a.in_base && ge < a.in_valid_end) ? load_word<FMT>(a.in, ge - a.in_base, ge, tune_step) : 0u;
                 }
             }
 #pragma unroll
@@ -384,7 +385,7 @@ fir1_tiled_kernel(const ScreenArgs sa, const TapsParam<T> taps, const FmaBand ba
 // group's windows cover are read once (ten 16-byte loads when the input is 16-byte aligned), converted once and kept in
 // registers; 8 outputs = 16 independent exact accumulator chains per thread.
 template <int T, int FMT>
-__global__ void __launch_bounds__(128) fir1_refine_group_kernel(const ScreenArgs sa, const TapsParam<T> taps)
+__global__ void __launch_bounds__(128) fir1_refine_group_kernel(const ScreenArgs sa, const TapsParam<T> taps, const uint32_t tune_step)
 {
     static_assert(T == 32, "window of 8 outputs = 39 samples, fetched as 40");
     const TiledArgs &a = sa.t;
@@ -400,7 +401,7 @@ __global__ void __launch_bounds__(128) fir1_refine_group_kernel(const ScreenArgs
 #pragma unroll
             for (int v = 0; v < (T + 8) / VS; v++) {
                 uint32_t x[VS];
-                load_words16<FMT>(a.in, (g0 - a.in_base) + VS * v, x);
+                load_words16<FMT>(a.in, (g0 - a.in_base) + VS * v, g0 + VS * v, tune_step, x);
 #pragma unroll
                 for (int e = 0; e < VS; e++) win[VS * v + e] = sc16q11_to_float2(x[e]);
             }
@@ -408,7 +409,7 @@ __global__ void __launch_bounds__(128) fir1_refine_group_kernel(const ScreenArgs
 #pragma unroll
             for (int q = 0; q < T + 8; q++) {
                 const i64 g = g0 + q;
-                win[q] = sc16q11_to_float2((g >= 0 && g >= a.in_base && g < a.in_valid_end) ? load_word<FMT>(a.in, g - a.in_base) : 0u);
+                win[q] = sc16q11_to_float2((g >= 0 && g >= a.in_base && g < a.in_valid_end) ? load_word<FMT>(a.in, g - a.in_base, g, tune_step) : 0u);
             }
         }
         float re[8], im[8];
@@ -464,7 +465,8 @@ struct Taps2Param {
 constexpr int F2X_NT = 288, F2X_M = 512, F2X_IN = 4 * F2X_M + 80, F2X_NS = 2 * F2X_M + 30;
 
 template <bool FMA, bool ADAPT, int FMT>
-__global__ void __launch_bounds__(F2X_NT, 2) fir2_tiled_kernel(const ScreenArgs sa, const Taps2Param taps, const FmaBand band)
+__global__ void __launch_bounds__(F2X_NT, 2) fir2_tiled_kernel(const ScreenArgs sa, const Taps2Param taps, const FmaBand band,
+                                                                const uint32_t tune_step)
 {
     __shared__ float2 s_x[F2X_IN + F2X_IN / 8 + 8];        // (+8: the last phase-1 thread reads a few slots past its valid window)
     __shared__ float2 s_s[(F2X_NS + 3) / 4 * 5 + 1];
@@ -486,12 +488,12 @@ __global__ void __launch_bounds__(F2X_NT, 2) fir2_tiled_kernel(const ScreenArgs 
         const i64 g = g0 + VS * q;
         uint32_t w[VS];
         if (aligned && g >= a.in_base && g >= 0 && g + VS <= a.in_valid_end) {
-            load_words16<FMT>(a.in, g - a.in_base, w);
+            load_words16<FMT>(a.in, g - a.in_base, g, tune_step, w);
         } else {
 #pragma unroll
             for (int e = 0; e < VS; e++) {
                 const i64 ge = g + e;
-                w[e] = (ge >= 0 && ge >= a.in_base && ge < a.in_valid_end) ? load_word<FMT>(a.in, ge - a.in_base) : 0u;
+                w[e] = (ge >= 0 && ge >= a.in_base && ge < a.in_valid_end) ? load_word<FMT>(a.in, ge - a.in_base, ge, tune_step) : 0u;
             }
         }
 #pragma unroll
@@ -608,7 +610,7 @@ __global__ void __launch_bounds__(F2X_NT, 2) fir2_tiled_kernel(const ScreenArgs 
 // the reference's order j = 0, 1, ... (src/fir.c:313-318), so all sums stay bit-exact; 4.4x fewer MACs than the
 // lane-per-output form.
 template <int FMT>
-__global__ void __launch_bounds__(128) fir2_refine_group_kernel(const ScreenArgs sa, const Taps2Param taps)
+__global__ void __launch_bounds__(128) fir2_refine_group_kernel(const ScreenArgs sa, const Taps2Param taps, const uint32_t tune_step)
 {
     const TiledArgs &a = sa.t;
     const uint32_t n_groups = min(*sa.work_count, sa.work_cap);
@@ -620,8 +622,8 @@ __global__ void __launch_bounds__(128) fir2_refine_group_kernel(const ScreenArgs
         const i64 g_bot = 2 * (u_top - 45) + 1 - 15;           // oldest input: 4 m0 - 74
         const bool inside = g_bot >= a.in_base && g_bot >= 0 && g_top < a.in_valid_end;
         auto sample = [&](i64 g) -> float2 {
-            if (inside) return sc16q11_to_float2(load_word<FMT>(a.in, g - a.in_base));
-            return sc16q11_to_float2((g >= 0 && g >= a.in_base && g < a.in_valid_end) ? load_word<FMT>(a.in, g - a.in_base) : 0u);
+            if (inside) return sc16q11_to_float2(load_word<FMT>(a.in, g - a.in_base, g, tune_step));
+            return sc16q11_to_float2((g >= 0 && g >= a.in_base && g < a.in_valid_end) ? load_word<FMT>(a.in, g - a.in_base, g, tune_step) : 0u);
         };
         float2 w[16];                                          // w[k] = x[2u+1-k] for the current u
 #pragma unroll

@@ -13,6 +13,7 @@
 #include <cmath>
 #include <algorithm>
 #include <cstring>
+#include <mutex>
 #include <thread>
 #include <type_traits>
 #include <vector>
@@ -41,6 +42,23 @@ struct Stage {
 
 enum FirPath { FIR_GENERIC = 0, FIR_TILED_1STAGE_32, FIR_SCREEN_DEC4 };
 
+// The rotation table of tuned handles (input_fmt.cuh, tune_pairs), packed from ookd_tune_quarter once per device: the
+// values never change, so the first tuned handle on a device writes them before any tuned kernel can run there.
+cudaError_t upload_tune_table(int dev)
+{
+    static std::mutex mu;
+    static bool done[64];
+    std::lock_guard<std::mutex> lock(mu);
+    if (dev >= 0 && dev < 64 && done[dev]) return cudaSuccess;
+    uint32_t pairs[129];
+    for (int m = 0; m <= 128; m++) {
+        pairs[m] = (uint16_t) ookd_tune_quarter[m] | ((uint32_t) (uint16_t) ookd_tune_quarter[256 - m] << 16);
+    }
+    const cudaError_t e = cudaMemcpyToSymbol(tune_pairs, pairs, sizeof(pairs));
+    if (e == cudaSuccess && dev >= 0 && dev < 64) done[dev] = true;
+    return e;
+}
+
 }  // namespace
 
 struct ookd_gpu {
@@ -65,8 +83,9 @@ struct ookd_gpu {
     uint32_t burst_rounds = 1;
     bool burst_fixed = false;         // sm_burst_rounds given in the configuration: no adaptation
     uint32_t flags = 0;
-    int fmt = FMT_SC16Q11;            // capture format (OOKD_FLAG_INPUT_*, input_fmt.cuh)
+    int fmt = FMT_SC16Q11;            // capture format (OOKD_FLAG_INPUT_*, input_fmt.cuh), + FMT_TUNED with a tune step
     uint32_t in_bytes = 4;            // ... its bytes per sample
+    uint32_t tune_step = 0;           // cfg.tune_step (ookd_gpu.h, "Tuning"); kernels ignore it unless fmt is tuned
     bool screen = false;
     bool screen2 = false;             // dec4 shape: screen + refine (else the exact tiled two-stage kernel)
     bool fma = false;                 // FMA screening (fused multiply-add pass + rigorous band, exact refine of the band):
@@ -332,20 +351,27 @@ encode_tiled_fn tensor_map_encoder()
 }
 
 // Calls f(std::integral_constant<int, FMT>) for the handle's capture format: every kernel that reads the capture is
-// instantiated per format (input_fmt.cuh).
+// instantiated per format, tuned or not (input_fmt.cuh).
 template <typename F>
 void with_fmt(int fmt, F &&f)
 {
-    if (fmt == FMT_CS8) {
-        f(std::integral_constant<int, FMT_CS8>());
-    } else if (fmt == FMT_CU8) {
-        f(std::integral_constant<int, FMT_CU8>());
-    } else {
-        f(std::integral_constant<int, FMT_SC16Q11>());
+    switch (fmt) {
+    case FMT_CS8: f(std::integral_constant<int, FMT_CS8>()); break;
+    case FMT_CU8: f(std::integral_constant<int, FMT_CU8>()); break;
+    case FMT_SC16Q11 | FMT_TUNED: f(std::integral_constant<int, FMT_SC16Q11 | FMT_TUNED>()); break;
+    case FMT_CS8 | FMT_TUNED: f(std::integral_constant<int, FMT_CS8 | FMT_TUNED>()); break;
+    case FMT_CU8 | FMT_TUNED: f(std::integral_constant<int, FMT_CU8 | FMT_TUNED>()); break;
+    default: f(std::integral_constant<int, FMT_SC16Q11>()); break;
     }
 }
 
-typedef void (*screen_tma_kernel_t)(const CUtensorMap, const ScreenTmaArgs, const ScreenParams);
+typedef void (*screen_tma_kernel_t)(const CUtensorMap, const ScreenTmaArgs, const ScreenParams, const uint32_t);
+
+// dynamic shared memory of the screening kernel: tuned formats keep the rotation table behind the mbarriers
+size_t screen_tma_smem(int fmt)
+{
+    return STMA_SMEM_BYTES + (fmt_tuned(fmt) ? STMA_TUNE_BYTES : 0);
+}
 
 screen_tma_kernel_t screen_tma_fn(int dec, bool adapt, int fmt)
 {
@@ -442,7 +468,8 @@ int launch_screen_tma(ookd_gpu *h, const ScreenArgs &sa, const ScreenParams &sp,
     cudaEvent_t *tok = (share && use_token) ? screen_token(h->device) : nullptr;
     if (tok) CU(h, cudaStreamWaitEvent(h->s_compute, *tok, 0));
     const unsigned grid = (unsigned) (tiles < ctas ? tiles : ctas);
-    screen_tma_fn(dec, h->adaptive, h->fmt)<<<grid, STMA_NT, STMA_SMEM_BYTES, h->s_compute>>>(tmap, ta, sp);
+    screen_tma_fn(dec, h->adaptive, h->fmt)<<<grid, STMA_NT, screen_tma_smem(h->fmt), h->s_compute>>>(tmap, ta, sp,
+                                                                                                  h->tune_step);
     if (tok) CU(h, cudaEventRecord(*tok, h->s_compute));
     return OOKD_OK;
 }
@@ -476,11 +503,11 @@ int launch_fir(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_valid_end,
             with_fmt(h->fmt, [&](auto fc) {
                 constexpr int FMT = decltype(fc)::value;
                 if (h->adaptive) {
-                    fir1_tiled_kernel<32, TILE_R, true, true, FMT><<<(unsigned) tiles, 256, 0, h->s_compute>>>(sa, tp, band);
+                    fir1_tiled_kernel<32, TILE_R, true, true, FMT><<<(unsigned) tiles, 256, 0, h->s_compute>>>(sa, tp, band, h->tune_step);
                 } else if (h->fma) {
-                    fir1_tiled_kernel<32, TILE_R, true, false, FMT><<<(unsigned) tiles, 256, 0, h->s_compute>>>(sa, tp, band);
+                    fir1_tiled_kernel<32, TILE_R, true, false, FMT><<<(unsigned) tiles, 256, 0, h->s_compute>>>(sa, tp, band, h->tune_step);
                 } else {
-                    fir1_tiled_kernel<32, TILE_R, false, false, FMT><<<(unsigned) tiles, 256, 0, h->s_compute>>>(sa, tp, band);
+                    fir1_tiled_kernel<32, TILE_R, false, false, FMT><<<(unsigned) tiles, 256, 0, h->s_compute>>>(sa, tp, band, h->tune_step);
                 }
             });
         }
@@ -516,11 +543,11 @@ int launch_fir(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_valid_end,
         with_fmt(h->fmt, [&](auto fc) {
             constexpr int FMT = decltype(fc)::value;
             if (h->adaptive) {
-                fir2_tiled_kernel<true, true, FMT><<<(unsigned) tiles, F2X_NT, 0, h->s_compute>>>(sa, tp, band);
+                fir2_tiled_kernel<true, true, FMT><<<(unsigned) tiles, F2X_NT, 0, h->s_compute>>>(sa, tp, band, h->tune_step);
             } else if (h->fma) {
-                fir2_tiled_kernel<true, false, FMT><<<(unsigned) tiles, F2X_NT, 0, h->s_compute>>>(sa, tp, band);
+                fir2_tiled_kernel<true, false, FMT><<<(unsigned) tiles, F2X_NT, 0, h->s_compute>>>(sa, tp, band, h->tune_step);
             } else {
-                fir2_tiled_kernel<false, false, FMT><<<(unsigned) tiles, F2X_NT, 0, h->s_compute>>>(sa, tp, band);
+                fir2_tiled_kernel<false, false, FMT><<<(unsigned) tiles, F2X_NT, 0, h->s_compute>>>(sa, tp, band, h->tune_step);
             }
         });
         h->launches++;
@@ -542,7 +569,7 @@ int launch_fir_refine(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_val
         tp.d_t2 = h->stages[1].d_taps;
         ScreenArgs sa = screen_args(h, d_in, in_base, in_valid_end);
         with_fmt(h->fmt, [&](auto fc) {
-            fir2_refine_group_kernel<decltype(fc)::value><<<16 * h->n_sm, 128, 0, h->s_compute>>>(sa, tp);
+            fir2_refine_group_kernel<decltype(fc)::value><<<16 * h->n_sm, 128, 0, h->s_compute>>>(sa, tp, h->tune_step);
         });
         h->launches++;
         CU(h, cudaGetLastError());
@@ -553,7 +580,7 @@ int launch_fir_refine(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_val
     memcpy(tp.t, h->stages[0].taps.data(), sizeof(tp.t));
     ScreenArgs sa = screen_args(h, d_in, in_base, in_valid_end);
     with_fmt(h->fmt, [&](auto fc) {
-        fir1_refine_group_kernel<32, decltype(fc)::value><<<16 * h->n_sm, 128, 0, h->s_compute>>>(sa, tp);
+        fir1_refine_group_kernel<32, decltype(fc)::value><<<16 * h->n_sm, 128, 0, h->s_compute>>>(sa, tp, h->tune_step);
     });
     h->launches++;
     CU(h, cudaGetLastError());
@@ -617,10 +644,10 @@ int run_generic_chain(ookd_gpu *h, const void *d_in, bool in_is_i16, i64 in_base
         const size_t smem = st.T * sizeof(float);
         if (src_i16) {
             with_fmt(h->fmt, [&](auto fc) {
-                fir_stage_generic_kernel<true, decltype(fc)::value><<<grid, 256, smem, h->s_compute>>>(a);
+                fir_stage_generic_kernel<true, decltype(fc)::value><<<grid, 256, smem, h->s_compute>>>(a, h->tune_step);
             });
         } else {
-            fir_stage_generic_kernel<false, FMT_SC16Q11><<<grid, 256, smem, h->s_compute>>>(a);
+            fir_stage_generic_kernel<false, FMT_SC16Q11><<<grid, 256, smem, h->s_compute>>>(a, 0u);
         }
         h->launches++;
         CU(h, cudaGetLastError());
@@ -1517,6 +1544,8 @@ int ookd_gpu_create(ookd_gpu **out, const struct ookd_gpu_config *cfg)
     h->flags = cfg->flags;
     h->fmt = (cfg->flags & OOKD_FLAG_INPUT_CS8) ? FMT_CS8 : (cfg->flags & OOKD_FLAG_INPUT_CU8) ? FMT_CU8 : FMT_SC16Q11;
     h->in_bytes = h->fmt == FMT_SC16Q11 ? 4 : 2;
+    h->tune_step = cfg->tune_step;
+    if (h->tune_step) h->fmt |= FMT_TUNED;               // step 0: the untuned kernels, exactly
     h->chunk_buffers = cfg->sm_chunk_buffers ? cfg->sm_chunk_buffers : 64;
     h->warmup = cfg->sm_warmup != 0 || (cfg->sub_windows > 1 && cfg->sm);
     h->burst_rounds = cfg->sm_burst_rounds ? (cfg->sm_burst_rounds < 16 ? cfg->sm_burst_rounds : 16) : FAST_BURST_ROUNDS;
@@ -1528,6 +1557,7 @@ int ookd_gpu_create(ookd_gpu **out, const struct ookd_gpu_config *cfg)
     do { if ((call) != cudaSuccess) { CREATE_FAIL(OOKD_ERR_CUDA); } } while (0)
 
     CUC(cudaSetDevice(dev));
+    if (h->tune_step && upload_tune_table(dev) != cudaSuccess) CREATE_FAIL(OOKD_ERR_CUDA);
     CUC(cudaStreamCreateWithFlags(&h->s_compute, cudaStreamNonBlocking));
     CUC(cudaStreamCreateWithFlags(&h->s_copy, cudaStreamNonBlocking));
     CUC(cudaEventCreate(&h->ev_t0));
@@ -1621,7 +1651,7 @@ int ookd_gpu_create(ookd_gpu **out, const struct ookd_gpu_config *cfg)
         for (int dec : {1, 4}) {
             for (bool adapt : {false, true}) {
                 if (cudaFuncSetAttribute(screen_tma_fn(dec, adapt, h->fmt), cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         STMA_SMEM_BYTES) != cudaSuccess) {
+                                         (int) screen_tma_smem(h->fmt)) != cudaSuccess) {
                     cudaGetLastError();
                     CREATE_FAIL(OOKD_ERR_CUDA);
                 }
@@ -1774,7 +1804,7 @@ int ookd_gpu_decode_begin(ookd_gpu *h, const int16_t *iq, int iq_is_device_ptr, 
         pa.out_lo = h->bit_base; pa.out_hi = o_hi_probe;
         with_fmt(h->fmt, [&](auto fc) {
             screen_probe_kernel<decltype(fc)::value><<<1, 1024, 0, h->s_compute>>>(
-                pa, (int) h->total_dec, (int) h->halo_fir + 1, sp.k0, (uint32_t *) ((char *) h->scalars.p + 344));
+                pa, (int) h->total_dec, (int) h->halo_fir + 1, sp.k0, (uint32_t *) ((char *) h->scalars.p + 344), h->tune_step);
         });
         h->launches++;
         CU(h, cudaGetLastError());

@@ -32,6 +32,11 @@
 // l>>2 of that block and forms its statistics straight from the bytes (screen_span_stats8); the prefix rows written in
 // place then overwrite only the warp's own raw bytes, so a __syncwarp (not a CTA barrier) separates the raw reads from
 // the prefix writes.  Shared memory, the 3-stage ring and 4 CTAs/SM stay as they are (DESIGN section 3.9).
+//
+// Tuned formats (FMT_TUNED, input_fmt.cuh): the copies and the ring are those of the untuned format; each thread rotates
+// its 16 words in registers right after the LDS (an 8-bit span is widened first and then takes the word statistics,
+// screen_span_stats_v2: dp4a on bytes does not apply to rotated words).  The 129 table pairs sit behind the mbarriers in
+// shared memory (STMA_TUNE_BYTES, inside the budget of four CTAs per SM; DESIGN section 3.10).
 #pragma once
 
 #include <cuda.h>
@@ -55,7 +60,8 @@ constexpr int STMA_HIST = 384;                                  // bytes of hist
 constexpr int STMA_XY_ROWS = STMA_NT + STMA_HT_MAX;
 // bodies | history rows | (sum I, sum Q) rows | mbarriers
 constexpr int STMA_SMEM_BYTES = STMA_STAGES * STMA_BODY + STMA_STAGES * STMA_HIST + STMA_STAGES * STMA_XY_ROWS * 8 + 32;
-static_assert(4 * (STMA_SMEM_BYTES + 1024) <= 228 * 1024, "four CTAs per SM");
+constexpr int STMA_TUNE_BYTES = 528;                            // tuned formats: tune_pairs (129 x 4 B), rounded to 16 B
+static_assert(4 * (STMA_SMEM_BYTES + STMA_TUNE_BYTES + 1024) <= 228 * 1024, "four CTAs per SM");
 
 #ifndef OOKD_STMA_L2_HINT
 #define OOKD_STMA_L2_HINT 0x12F0000000000000ull     /* evict-first (0x1000000000000000 = normal, 0x14F0000000000000 = evict-last) */
@@ -246,13 +252,14 @@ __device__ __forceinline__ void screen_span_stats8(const uint32_t (&x)[8], uint3
 // registers and the kernel measures 4 % faster)
 template <int DEC, bool ADAPT, int FMT>
 __global__ void __maxnreg__(64)
-fir_screen_tma_kernel(const __grid_constant__ CUtensorMap tmap, const ScreenTmaArgs ta, const ScreenParams sp)
+fir_screen_tma_kernel(const __grid_constant__ CUtensorMap tmap, const ScreenTmaArgs ta, const ScreenParams sp,
+                      const uint32_t tune_step)
 {
     static_assert(DEC == 1 || DEC == 4, "shapes with a screening proof");
     constexpr int NT = STMA_NT, SPT = STMA_SPT, L = STMA_L, NS = STMA_STAGES;
     constexpr int HT = (DEC == 1) ? 2 : 5;                     // history spans
     constexpr int LOUT = L / DEC;                              // outputs per tile
-    constexpr int LOG_RS = (FMT == FMT_SC16Q11) ? 5 : 6;       // samples per 128-byte tensor row: 32 or 64
+    constexpr int LOG_RS = (fmt_raw(FMT) == FMT_SC16Q11) ? 5 : 6;   // samples per 128-byte tensor row: 32 or 64
     extern __shared__ __align__(1024) uint8_t smem_raw[];
 
     const ScreenArgs &sa = ta.s;
@@ -273,12 +280,16 @@ fir_screen_tma_kernel(const __grid_constant__ CUtensorMap tmap, const ScreenTmaA
     const uint32_t hist0 = body0 + NS * STMA_BODY + STMA_HIST;   // + STMA_HIST: history rows are rows -3..-1 of their stage
     const uint32_t xy0 = body0 + NS * STMA_BODY + NS * STMA_HIST;
     const uint32_t bar0 = xy0 + NS * STMA_XY_ROWS * 8;
+    const uint32_t tab0 = bar0 + 32;                             // tuned formats: tune_pairs
 
     const int u = (int) threadIdx.x;
     if (u == 0) {
 #pragma unroll
         for (int s = 0; s < NS; s++) mbar_init(bar0 + 8 * s, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if constexpr (fmt_tuned(FMT)) {
+        if (u < 129) asm volatile("st.shared.u32 [%0], %1;" ::"r"(tab0 + 4 * u), "r"(__ldg(tune_pairs + u)) : "memory");
     }
     __syncthreads();
 
@@ -288,7 +299,7 @@ fir_screen_tma_kernel(const __grid_constant__ CUtensorMap tmap, const ScreenTmaA
     auto issue = [&](uint32_t tile, int s) {
         const uint32_t bar = bar0 + 8 * s;
         mbar_expect_tx(bar, L * in_bytes<FMT>());
-        if constexpr (FMT == FMT_SC16Q11) {
+        if constexpr (fmt_raw(FMT) == FMT_SC16Q11) {
             tma_load_tile(body0 + s * STMA_BODY, &tmap, tile_row(tile), bar);
         } else {
 #pragma unroll
@@ -301,7 +312,18 @@ fir_screen_tma_kernel(const __grid_constant__ CUtensorMap tmap, const ScreenTmaA
 #pragma unroll
         for (int e = 0; e < 16; e++) {
             const i64 ge = g + e;
-            w[e] = (ge >= 0 && ge >= a.in_base && ge < a.in_valid_end) ? load_word<FMT>(a.in, ge - a.in_base) : 0u;
+            w[e] = (ge >= 0 && ge >= a.in_base && ge < a.in_valid_end) ? load_word<FMT>(a.in, ge - a.in_base, ge, tune_step) : 0u;
+        }
+    };
+    // tuned formats: the 16 words of the span starting at global sample g, as loaded from the ring, rotated in place
+    auto tune_span = [&](i64 g, uint32_t (&w)[16]) {
+        const uint32_t phi0 = (uint32_t) g * tune_step;
+#pragma unroll
+        for (int e = 0; e < 16; e++) {
+            const uint32_t phi = phi0 + (uint32_t) e * tune_step;
+            uint32_t pair;
+            asm volatile("ld.shared.u32 %0, [%1];" : "=r"(pair) : "r"(tab0 + 4 * tune_row(phi)));
+            w[e] = tune_rotate(w[e], phi, pair);
         }
     };
     // base address of the row of virtual thread uu (>= 0: body, < 0: history rows) of stage s
@@ -347,7 +369,7 @@ fir_screen_tma_kernel(const __grid_constant__ CUtensorMap tmap, const ScreenTmaA
         const i64 o0 = a.out_lo + (i64) tile * LOUT;
         uint32_t pre[SPT], tot_own;                                         // tot_own bit 31 = "span out of range"
         int sx, sy;
-        if constexpr (FMT == FMT_SC16Q11) {
+        if constexpr (fmt_raw(FMT) == FMT_SC16Q11) {
             uint32_t w[16];
             if (tile_fast(tile)) {
                 mbar_wait(bar0 + 8 * s, (phases >> s) & 1u);
@@ -357,6 +379,7 @@ fir_screen_tma_kernel(const __grid_constant__ CUtensorMap tmap, const ScreenTmaA
                     const uint4 x = lds128(body + off_own[v]);
                     w[4 * v] = x.x; w[4 * v + 1] = x.y; w[4 * v + 2] = x.z; w[4 * v + 3] = x.w;
                 }
+                if constexpr (fmt_tuned(FMT)) tune_span(tile_in0(tile) + (i64) u * SPT, w);
             } else {
                 load_span_slow(tile_in0(tile) + (i64) u * SPT, w);
             }
@@ -367,13 +390,24 @@ fir_screen_tma_kernel(const __grid_constant__ CUtensorMap tmap, const ScreenTmaA
                 phases ^= 1u << s;
                 const int r = (u & 31) >> 2;                     // raw row of 64 samples in the warp's block; chunks 2(u&3), 2(u&3)+1
                 const uint32_t blk = body + 2048 * (u >> 5);
-                uint32_t x[8];
+                if constexpr (fmt_tuned(FMT)) {
+                    uint32_t w[16];
 #pragma unroll
-                for (int v = 0; v < 2; v++) {
-                    const uint4 c = lds128(blk + r * 128 + ((((u & 3) << 1 | v) ^ r) << 4));
-                    x[4 * v] = c.x; x[4 * v + 1] = c.y; x[4 * v + 2] = c.z; x[4 * v + 3] = c.w;
+                    for (int v = 0; v < 2; v++) {
+                        uint32_t (&w8)[8] = *reinterpret_cast<uint32_t (*)[8]>(w + 8 * v);
+                        widen8x8<fmt_raw(FMT)>(lds128(blk + r * 128 + ((((u & 3) << 1 | v) ^ r) << 4)), w8);
+                    }
+                    tune_span(tile_in0(tile) + (i64) u * SPT, w);
+                    screen_span_stats_v2(w, pre, sx, sy, tot_own, sp.k0);
+                } else {
+                    uint32_t x[8];
+#pragma unroll
+                    for (int v = 0; v < 2; v++) {
+                        const uint4 c = lds128(blk + r * 128 + ((((u & 3) << 1 | v) ^ r) << 4));
+                        x[4 * v] = c.x; x[4 * v + 1] = c.y; x[4 * v + 2] = c.z; x[4 * v + 3] = c.w;
+                    }
+                    screen_span_stats8<FMT>(x, pre, sx, sy, tot_own, sp.k0);
                 }
-                screen_span_stats8<FMT>(x, pre, sx, sy, tot_own, sp.k0);
             } else {
                 uint32_t w[16];
                 load_span_slow(tile_in0(tile) + (i64) u * SPT, w);

@@ -4,10 +4,12 @@
  *
  * Supported SDR types: bladerf_file (SC16Q11 capture files), and for --rx also cu8_file (RTL-SDR, uint8 I,Q) and
  * cs8_file (HackRF / bladeRF SC8_Q7, int8 I,Q), decoded natively on the GPU.  Options that only configure live
- * bladeRF hardware (frequency, bandwidth, gain, stream sizing) are accepted and ignored.
+ * bladeRF hardware (frequency, bandwidth, gain, stream sizing) are accepted and ignored: a file's centre frequency is
+ * fixed, and --rx-offset tunes to a transmitter away from it.
  */
 #include <getopt.h>
 #include <limits.h>
+#include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -27,6 +29,7 @@
 #define OPT_GPUS 0x252
 #define OPT_WINDOW 0x253
 #define OPT_GPU_IDS 0x254
+#define OPT_RX_OFFSET 0x255
 
 static const struct option long_options[] = {
     { "rx", required_argument, 0, 'r' },
@@ -41,6 +44,7 @@ static const struct option long_options[] = {
     { "rx-rec-dig", required_argument, 0, 'B' },
     { "rx-filter", required_argument, 0, 'F' },
     { "rx-fmt", required_argument, 0, OPT_RX_FMT },
+    { "rx-offset", required_argument, 0, OPT_RX_OFFSET },
     { "sdr-args", required_argument, 0, 'A' },
     { "frequency", required_argument, 0, 'f' },
     { "samplerate", required_argument, 0, 's' },
@@ -80,7 +84,9 @@ static void usage(const char *argv0)
     printf("  -R, --rx-rec <[type,]file>    Record the filtered samples (SC16Q11) to a file.\n");
     printf("  --rx-rec-input                Record the input samples instead of the filtered ones.\n");
     printf("  -B, --rx-rec-dig <filename>   Save the digital signal transitions to a CSV file.\n");
-    printf("  --rx-fmt <fmt>                \"csv\" or \"pretty\" (default).\n\n");
+    printf("  --rx-fmt <fmt>                \"csv\" or \"pretty\" (default).\n");
+    printf("  --rx-offset <Hz>              Decode a transmitter this far from the capture's centre frequency\n");
+    printf("                                (signed, K/M/G suffixes allowed; below half the sample rate).\n\n");
     printf("SDR configuration options:\n");
     printf("  -A, --sdr-args <file>         Capture file (\"-\": stdin): SC16Q11 for bladerf_file, interleaved\n");
     printf("                                uint8 I,Q for cu8_file, int8 I,Q for cs8_file.\n");
@@ -116,6 +122,23 @@ static bool parse_rate(const char *s, unsigned int *out)    /* str2uint_suffix, 
     return true;
 }
 
+/* --rx-offset: a signed frequency with the suffixes of parse_rate */
+static bool parse_offset(const char *s, double *out)
+{
+    char *end;
+    const double v = strtod(s, &end);
+    double mult = 1;
+    if (end == s || !isfinite(v)) {
+        return false;
+    }
+    if (!strcasecmp(end, "K") || !strcasecmp(end, "KHz")) mult = 1e3;
+    else if (!strcasecmp(end, "M") || !strcasecmp(end, "MHz")) mult = 1e6;
+    else if (!strcasecmp(end, "G") || !strcasecmp(end, "GHz")) mult = 1e9;
+    else if (*end != '\0') return false;
+    *out = v * mult;
+    return isfinite(*out);
+}
+
 static bool parse_level(const char *s, enum ookd_log_level *out)
 {
     static const char *names[] = { "verbose", "debug", "info", "warning", "error", "critical", "silent" };
@@ -134,6 +157,8 @@ int main(int argc, char *argv[])
     struct ookd_keyval_list params;
     int direction = -1;         /* 0 rx, 1 tx */
     bool have_fmt = false;
+    const char *offset_arg = NULL;
+    double offset_hz = 0.0;
     int c, idx;
 
     ookd_cfg_init(&cfg);
@@ -233,6 +258,13 @@ int main(int argc, char *argv[])
                 }
                 have_fmt = true;
                 break;
+            case OPT_RX_OFFSET:
+                if (!parse_offset(optarg, &offset_hz)) {
+                    fprintf(stderr, "Invalid RX offset: %s\n", optarg);
+                    return EXIT_FAILURE;
+                }
+                offset_arg = optarg;
+                break;
             case 'A': cfg.sdr_args = optarg; break;
             case 's':
                 if (!parse_rate(optarg, &cfg.samplerate)) {
@@ -303,6 +335,11 @@ int main(int argc, char *argv[])
     }
 
     int status;
+    if (offset_arg && direction == 0 && ookd_tune_step(offset_hz, cfg.samplerate, &cfg.tune_step) != OOKD_OK) {
+        fprintf(stderr, "Error: RX offset %s is out of range: it must be below half the sample rate (%u Hz) in "
+                "magnitude.\n", offset_arg, cfg.samplerate / 2);
+        return EXIT_FAILURE;
+    }
     if (direction == 0) {
         if (!cfg.device && !cfg.rx_rec_dig && !cfg.rx_rec) {    /* validate_cfg, src/main.c:244-283 */
             fprintf(stderr, "Error: Either a target device or recording parameters must be specified.\n");
@@ -320,6 +357,10 @@ int main(int argc, char *argv[])
         }
         if (cfg.rx_filter) {
             fprintf(stderr, "Error: --rx-filter cannot be used with --tx.\n");
+            return EXIT_FAILURE;
+        }
+        if (offset_arg) {
+            fprintf(stderr, "Error: --rx-offset cannot be used with --tx.\n");
             return EXIT_FAILURE;
         }
         status = ookd_tx(&cfg);

@@ -118,6 +118,8 @@ struct ookd_cfg {                       /* the fields of struct ookiedokie_cfg t
     FILE    *out;                       /* message output, NULL => stdout                     */
     uint32_t input_flags;               /* capture format: 0 SC16Q11 (bladerf_file), OOKD_FLAG_INPUT_CS8 (cs8_file) or
                                            OOKD_FLAG_INPUT_CU8 (cu8_file); recordings stay SC16Q11  */
+    uint32_t tune_step;                 /* --rx-offset as ookd_gpu_config.tune_step (0: off); --rx-rec-input then
+                                           records the tuned samples the decode saw                                */
 };
 void ookd_cfg_init(struct ookd_cfg *cfg);               /* defaults of src/ookiedokie_cfg.c:27-38 */
 int  ookd_rx(const struct ookd_cfg *cfg);               /* 0 on success */

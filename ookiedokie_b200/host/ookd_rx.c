@@ -250,16 +250,18 @@ static int write_rec_filtered(struct rx_out *o, ookd_gpu *gpu)
 /* --rx-rec-input (src/ookiedokie.c:248-253): the raw buffers, the last one zero padded like sdr_bladerf_file_rx
  * leaves it (int16 -> float -> (int16_t)(x * 2048.0f) is the identity).  The recording is an SC16Q11 file whatever the
  * capture's format: 8-bit samples are written widened (CS8 k -> 16 k, CU8 v -> 16 v - 2040, the value they stand
- * for), and the padding is SC16Q11 zeros. */
-static int write_rec_input(struct rx_out *o, const struct rx_slot *s, uint64_t halo, uint64_t spb, uint32_t input_flags)
+ * for), and the padding is SC16Q11 zeros.  With a tune step the samples are written tuned (ookd_tune_sc16q11, at their
+ * global index): the recording is the capture the decode saw, and decodes untuned to the same output. */
+static int write_rec_input(struct rx_out *o, const struct rx_slot *s, uint64_t halo, uint64_t spb, uint32_t input_flags,
+                           uint32_t tune_step)
 {
-    if (!input_flags) {
+    if (!input_flags && !tune_step) {
         if (fwrite(s->buf + 4 * (size_t) halo, 4, s->have, o->rec) != s->have) {
             log_error("Sample file write was truncated.\n");
             return OOKD_ERR_STATE;
         }
     } else {
-        const uint8_t *src = s->buf + 2 * (size_t) halo;
+        const uint8_t *src = s->buf + (input_flags ? 2 : 4) * (size_t) halo;
         const size_t step = 1u << 16;
         if (o->rec_cap < step) {
             free(o->rec_buf);
@@ -271,9 +273,16 @@ static int write_rec_input(struct rx_out *o, const struct rx_slot *s, uint64_t h
         }
         for (size_t i0 = 0; i0 < s->have; i0 += step) {
             const size_t n = s->have - i0 < step ? s->have - i0 : step;
-            for (size_t k = 0; k < 2 * n; k++) {
-                const uint8_t b = src[2 * i0 + k];
-                o->rec_buf[k] = (input_flags & OOKD_FLAG_INPUT_CS8) ? (int16_t) (16 * (int8_t) b) : (int16_t) (16 * b - 2040);
+            if (!input_flags) {
+                memcpy(o->rec_buf, src + 4 * i0, 4 * n);
+            } else {
+                for (size_t k = 0; k < 2 * n; k++) {
+                    const uint8_t b = src[2 * i0 + k];
+                    o->rec_buf[k] = (input_flags & OOKD_FLAG_INPUT_CS8) ? (int16_t) (16 * (int8_t) b) : (int16_t) (16 * b - 2040);
+                }
+            }
+            if (tune_step) {
+                ookd_tune_sc16q11(o->rec_buf, o->rec_buf, s->first_sample + i0, n, tune_step);
             }
             if (fwrite(o->rec_buf, 4, n, o->rec) != n) {
                 log_error("Sample file write was truncated.\n");
@@ -366,6 +375,7 @@ int ookd_rx(const struct ookd_cfg *cfg)
     gc.samples_per_buffer = cfg->samples_per_buffer;
     gc.device_id = cfg->gpu_id;
     gc.flags = cfg->input_flags;
+    gc.tune_step = cfg->tune_step;
     const unsigned n_gpus = cfg->n_gpus > 1 ? cfg->n_gpus : 1;
     int rc;
     uint32_t halo;
@@ -499,7 +509,7 @@ int ookd_rx(const struct ookd_cfg *cfg)
 
         if (o.rec) {
             if (rec_input) {
-                rc = write_rec_input(&o, cur, halo, spb, cfg->input_flags);
+                rc = write_rec_input(&o, cur, halo, spb, cfg->input_flags, cfg->tune_step);
             } else if (multi) {
                 rc = OOKD_OK;
                 for (uint32_t q = 0; rc == OOKD_OK && q < ookd_gpu_multi_shards_used(multi); q++) {

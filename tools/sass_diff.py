@@ -71,8 +71,9 @@ def build_rev(rev, tmp):
     os.makedirs(src)
     arch = subprocess.run(["git", "-C", ROOT, "archive", rev], check=True, capture_output=True).stdout
     subprocess.run(["tar", "-x", "-C", src], input=arch, check=True)
-    subprocess.run(["make", "-C", os.path.join(src, "ookiedokie_b200", "csrc"), os.path.abspath(
-        os.path.join(src, "ookiedokie_b200", "lib", "ookd_gpu.o"))], check=True, capture_output=True)
+    # (the Makefile names its targets relative to csrc/)
+    subprocess.run(["make", "-C", os.path.join(src, "ookiedokie_b200", "csrc"), "../lib/ookd_gpu.o"],
+                   check=True, capture_output=True)
     return os.path.join(src, "ookiedokie_b200", "lib", "ookd_gpu.o")
 
 
