@@ -161,6 +161,37 @@ int ookd_tune_step(double offset_hz, uint32_t samplerate, uint32_t *step);
  * out may equal in.  8-bit captures are widened to SC16Q11 words first. */
 int ookd_tune_sc16q11(const int16_t *in, int16_t *out, uint64_t first_sample, uint64_t n_samples, uint32_t step);
 
+/* ---- Levels: choose the on/off threshold from the capture's noise floor ----
+ * ookd_gpu_levels counts the filtered outputs of a span by their power; ookd_level_threshold turns the counts into a
+ * threshold.  Both are integer-exact, so a handle created with the threshold chosen decodes exactly as a handle given
+ * that float does.
+ *
+ *   Power.  p(o) = power_exact(re, im) = fl(fl(re*re) + fl(im*im)) of the filtered, decimated output o: the value the
+ *     threshold decision compares with P*.  It uses the handle's filter, its format (8-bit widened first) and its
+ *     tune_step (so it is the power of T(x)).
+ *   Bin.  bin(p) = (bits(p) & 0x7FFFFFFF) >> 19, OOKD_LEVEL_BINS = 4096 bins, 16 per octave of power: 0 through the
+ *     subnormals up to bin 4079; bin 4080 is +inf.  Bin b holds the powers in [f(b << 19), f((b + 1) << 19)), f(bits)
+ *     being the float with those bits.  Every NaN counts in bin 4088, the bin of the reference platform's default NaN
+ *     (x86: 0xFFC00000): which NaN an operation returns differs between processors, and the count must not.
+ *   Span.  Input samples [first_sample, first_sample + n_samples); first_sample must be a multiple of the total
+ *     decimation (else OOKD_ERR_ARG).  iq points at sample first_sample - min(ookd_gpu_halo(h), first_sample), as for
+ *     ookd_gpu_decode_shard, in the handle's format (bytes, any alignment, for CS8 / CU8), on the host or, with
+ *     iq_is_device_ptr != 0, on the handle's device.  The histogram counts exactly the outputs
+ *     ookd_gpu_decode_shard(..., last = 0) reports for the span, floor(n_samples / decimation) of them: no EOF
+ *     padding, history before sample 0 is word 0.  So the histograms of adjacent spans add up to their union's.
+ *     hist (OOKD_LEVEL_BINS counts, host memory) is overwritten.  The call runs its own kernels and leaves the last
+ *     decode's results (ookd_gpu_edges, _bits, _filtered_sc16q11) as they were.
+ *   Threshold rule (ookd_level_threshold, CPU only).  n = sum(hist) (OOKD_ERR_ARG if it exceeds 2^64 - 1).  The median
+ *     bin m is the smallest with cum(m) >= n - cum(m), cum(m) = hist[0] + ... + hist[m].  The floor is
+ *     F = f((m + 1) << 19), the upper edge of the median bin, as a double, and
+ *       threshold = (float) sqrt(F * pow(10.0, margin_db / 10.0)).
+ *     OOKD_ERR_ARG if n == 0, F is not finite (m >= 4079), margin_db is not finite, or the threshold is not finite.
+ *     Negative margins are allowed; OOKD_LEVEL_MARGIN_DB is the CLI's default.  floor_power (nullable) receives F.
+ * No entry point changes a live handle's threshold: create the decode handles once it is chosen. */
+#define OOKD_LEVEL_BINS       4096
+#define OOKD_LEVEL_MARGIN_DB  12.0
+int ookd_level_threshold(const uint64_t *hist, double margin_db, float *threshold, double *floor_power);
+
 /* ---- results ---- */
 struct ookd_msg {
     uint64_t out_sample;                     /* post-decimation index of the sample that
@@ -410,6 +441,10 @@ int  ookd_gpu_filtered(ookd_gpu *h, const int16_t *iq, uint64_t n_samples, int i
  * sdr_bladerf_file_tx (src/sdr/bladeRF_file.c:128-155): what --rx-rec writes (src/ookiedokie.c:265-270).  Interleaved
  * int16 I,Q.  Uses the decode's input again: device input must still be valid, host input is the handle's staged copy. */
 int  ookd_gpu_filtered_sc16q11(ookd_gpu *h, int16_t *out_host, uint64_t max_out, uint64_t *n_out);
+
+/* Level histogram of the span [first_sample, first_sample + n_samples): see "Levels" above. */
+int  ookd_gpu_levels(ookd_gpu *h, const int16_t *iq, int iq_is_device_ptr, uint64_t first_sample, uint64_t n_samples,
+                     uint64_t *hist);
 
 /* Same arithmetic on caller-supplied complex float input (what fir_test feeds
  * fir_filter_and_decimate, src/test/fir_test.c:246-275). */

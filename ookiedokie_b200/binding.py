@@ -17,6 +17,8 @@ LIB_PATH = os.environ.get("OOKD_GPU_LIB") or os.path.join(_HERE, "lib", "libookd
 MAX_STAGES = 8
 MSG_BYTES = 32
 K_INF = 0xFFFFFFFF
+LEVEL_BINS = 4096
+LEVEL_MARGIN_DB = 12.0
 
 FLAG_FORCE_GENERIC = 1
 FLAG_NO_SCREEN = 2
@@ -36,7 +38,7 @@ INPUT_FORMATS = {"sc16q11": (0, np.int16), "cs8": (FLAG_INPUT_CS8, np.int8), "cu
 # every symbol include/ookd_gpu.h declares
 EXPORTS = [
     "ookd_sm_compile", "ookd_sm_compiled_free", "ookd_sm_idle_carry", "ookd_power_threshold",
-    "ookd_tune_step", "ookd_tune_sc16q11",
+    "ookd_tune_step", "ookd_tune_sc16q11", "ookd_level_threshold", "ookd_gpu_levels",
     "ookd_gpu_device_count", "ookd_gpu_strerror", "ookd_gpu_last_error",
     "ookd_gpu_create", "ookd_gpu_destroy", "ookd_gpu_decode", "ookd_gpu_decode_shard",
     "ookd_gpu_decode_begin", "ookd_gpu_decode_end", "ookd_gpu_batch_decode",
@@ -169,6 +171,10 @@ def lib():
         L.ookd_tune_step.argtypes = [C.c_double, C.c_uint32, C.POINTER(C.c_uint32)]
         L.ookd_tune_sc16q11.restype = C.c_int
         L.ookd_tune_sc16q11.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32]
+        L.ookd_level_threshold.restype = C.c_int
+        L.ookd_level_threshold.argtypes = [C.c_void_p, C.c_double, C.POINTER(C.c_float), C.POINTER(C.c_double)]
+        L.ookd_gpu_levels.restype = C.c_int
+        L.ookd_gpu_levels.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_uint64, C.c_uint64, C.c_void_p]
         L.ookd_gpu_device_count.restype = C.c_int
         L.ookd_gpu_strerror.restype = C.c_char_p
         L.ookd_gpu_strerror.argtypes = [C.c_int]
@@ -356,6 +362,23 @@ def tune_sc16q11(iq, first_sample, step):
     if rc != 0:
         raise OokdError(f"ookd_tune_sc16q11: {lib().ookd_gpu_strerror(rc).decode()}")
     return out
+
+
+def level_threshold(hist, margin_db=LEVEL_MARGIN_DB):
+    """Threshold rule of include/ookd_gpu.h, "Levels": a level histogram (LEVEL_BINS counts) -> (threshold, floor_power),
+    the float to create decode handles with and F, the upper edge of the median bin.  ValueError where
+    ookd_level_threshold returns OOKD_ERR_ARG: no counts, a median in the inf / NaN bins, a non-finite margin or
+    threshold, or more counts than a uint64 holds."""
+    h = np.asarray(hist)
+    if h.shape != (LEVEL_BINS,) or (h.dtype.kind not in "ui") or (h.dtype.kind == "i" and (h < 0).any()):
+        raise ValueError(f"a level histogram is {LEVEL_BINS} non-negative integer counts")
+    h = np.ascontiguousarray(h, dtype=np.uint64)
+    thr, floor = C.c_float(), C.c_double()
+    if lib().ookd_level_threshold(C.c_void_p(h.ctypes.data), C.c_double(float(margin_db)), C.byref(thr),
+                                  C.byref(floor)) != 0:
+        raise ValueError(f"no threshold from this histogram ({int(h.sum(dtype=np.float64))} outputs) at a margin of "
+                         f"{margin_db} dB: it needs outputs, a finite median power, and a finite margin and result")
+    return float(thr.value), float(floor.value)
 
 
 def device_count():
@@ -553,6 +576,19 @@ class Gpu:
         out = np.empty((m.value, 2), dtype=np.int16)
         self._check(lib().ookd_gpu_filtered_sc16q11(self.h, out.ctypes.data, m.value, C.byref(m)), "ookd_gpu_filtered_sc16q11")
         return out
+
+    def levels(self, iq, first_sample=0, n_samples=None):
+        """Level histogram (include/ookd_gpu.h, "Levels") of input samples [first_sample, first_sample + n_samples):
+        iq is a capture of the handle's input format pointing at sample first_sample - min(halo, first_sample), as for
+        decode_shard, or (device_ptr, n) with n the samples present there.  n_samples defaults to all of them after the
+        history.  -> uint64 array of LEVEL_BINS counts."""
+        p, n, is_dev, keep = _as_ptr(iq, self.input_format)
+        if n_samples is None:
+            n_samples = n - min(self.halo, int(first_sample))
+        hist = np.zeros(LEVEL_BINS, dtype=np.uint64)
+        self._check(lib().ookd_gpu_levels(self.h, p, is_dev, int(first_sample), int(n_samples), hist.ctypes.data),
+                    "ookd_gpu_levels")
+        return hist
 
     def filter_cf(self, iq_f32):
         x = np.ascontiguousarray(iq_f32, dtype=np.float32).reshape(-1, 2)

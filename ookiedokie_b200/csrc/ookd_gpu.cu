@@ -24,6 +24,7 @@
 #include "edge_kernels.cuh"
 #include "sm_kernels.cuh"
 #include "synth_kernel.cuh"
+#include "level_kernels.cuh"
 
 using namespace ookd;
 
@@ -589,7 +590,7 @@ int launch_fir_refine(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_val
 
 // The work list overflowed (most of the capture is near the threshold): decide the whole range exactly.
 int run_generic_chain(ookd_gpu *h, const void *d_in, bool in_is_i16, i64 in_base, i64 in_valid_end, i64 o_lo, i64 o_hi,
-                      float2 *out_cf, uint32_t *bits, i64 bit_base);
+                      float2 *out_cf, uint32_t *bits, i64 bit_base, size_t n_stages = SIZE_MAX);
 
 int launch_fir_exact_all(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_valid_end)
 {
@@ -604,11 +605,12 @@ int launch_fir_exact_all(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_
 // ---- shape-agnostic chain: one launch per stage, intermediates in HBM ----
 // Computes final outputs [o_lo, o_hi); writes decisions (bits != null) and/or the final
 // stage's samples (out_cf != null, out_cf[0] <-> o_lo).  `in` is the capture in the handle's format (in_is_i16) or float2.
+// n_stages < the filter's stage count runs the first n_stages stages only: "final" is then stage n_stages' output.
 int run_generic_chain(ookd_gpu *h, const void *d_in, bool in_is_i16, i64 in_base, i64 in_valid_end,
-                      i64 o_lo, i64 o_hi, float2 *out_cf, uint32_t *bits, i64 bit_base)
+                      i64 o_lo, i64 o_hi, float2 *out_cf, uint32_t *bits, i64 bit_base, size_t n_stages)
 {
     if (o_hi <= o_lo) return OOKD_OK;
-    const size_t ns = h->stages.size();
+    const size_t ns = std::min(h->stages.size(), n_stages);
     // required output range per stage, walking backwards
     std::vector<i64> lo(ns), hi(ns);
     i64 need_lo = o_lo, need_hi = o_hi;
@@ -2183,6 +2185,19 @@ int ookd_gpu_bits(ookd_gpu *h, uint8_t *bits_out, uint64_t max_out, uint64_t *n_
     return OOKD_OK;
 }
 
+// The input of a call that runs its own kernels on the device: device input as it is, host input copied (on s_compute)
+// into tmp, which the caller releases.
+static int stage_input(ookd_gpu *h, const void *in, bool in_dev, size_t bytes, DevBuf &tmp, const void **d_in)
+{
+    *d_in = in;
+    if (in_dev) return OOKD_OK;
+    const int rc = ensure(h, tmp, bytes + 16);
+    if (rc) return rc;
+    if (bytes) CU(h, cudaMemcpyAsync(tmp.p, in, bytes, cudaMemcpyHostToDevice, h->s_compute));
+    *d_in = tmp.p;
+    return OOKD_OK;
+}
+
 static int filtered_common(ookd_gpu *h, const void *in, bool in_i16, bool in_dev, uint64_t n_samples, bool pad_spb,
                            float *out_iq_host, uint64_t max_out, uint64_t *n_out)
 {
@@ -2198,13 +2213,7 @@ static int filtered_common(ookd_gpu *h, const void *in, bool in_i16, bool in_dev
     DevBuf tmp_in, tmp_out;
     const void *d_in = in;
     const size_t esz = in_i16 ? h->in_bytes : 8;
-    if (!in_dev) {
-        if ((rc = ensure(h, tmp_in, n_samples * esz + 16))) return rc;
-        if (n_samples) {
-            CU(h, cudaMemcpyAsync(tmp_in.p, in, n_samples * esz, cudaMemcpyHostToDevice, h->s_compute));
-        }
-        d_in = tmp_in.p;
-    }
+    if ((rc = stage_input(h, in, in_dev, n_samples * esz, tmp_in, &d_in))) return rc;
     rc = ensure(h, tmp_out, lim * sizeof(float2));
     if (!rc) rc = run_generic_chain(h, d_in, in_i16, 0, (i64) n_samples, 0, (i64) lim, (float2 *) tmp_out.p, nullptr, 0);
     if (!rc) {
@@ -2252,6 +2261,82 @@ int ookd_gpu_filtered_sc16q11(ookd_gpu *h, int16_t *out_host, uint64_t max_out, 
     cudaStreamSynchronize(h->s_compute);
     release(cf);
     release(q);
+    return rc;
+}
+
+// One launch of level_hist_kernel: outputs [o_lo, o_hi) of the last stage, read from the capture (in_raw) or from the
+// float2 outputs of the stage before it, added to d_hist.
+static int launch_levels(ookd_gpu *h, const void *d_in, bool in_raw, i64 in_base, i64 in_valid_end, i64 o_lo, i64 o_hi,
+                         u64 *d_hist)
+{
+    const Stage &st = h->stages.back();
+    LevelArgs a{};
+    a.in = d_in; a.in_base = in_base; a.in_valid_end = in_valid_end;
+    a.taps = st.d_taps; a.T = st.T; a.D = st.D;
+    a.out_lo = o_lo; a.out_hi = o_hi;
+    a.hist = (unsigned long long *) d_hist;
+    const u64 n = (u64) (o_hi - o_lo);
+    u64 grid = std::min<u64>((n + LEVEL_NT - 1) / LEVEL_NT, 8ull * h->n_sm);
+    grid = std::max<u64>(grid, (n + LEVEL_CTA_MAX - 1) / LEVEL_CTA_MAX);     // each CTA counts fewer than 2^32 outputs
+    const size_t smem = st.T * sizeof(float);
+    if (in_raw) {
+        with_fmt(h->fmt, [&](auto fc) {
+            level_hist_kernel<true, decltype(fc)::value><<<(unsigned) grid, LEVEL_NT, smem, h->s_compute>>>(a, h->tune_step);
+        });
+    } else {
+        level_hist_kernel<false, FMT_SC16Q11><<<(unsigned) grid, LEVEL_NT, smem, h->s_compute>>>(a, 0u);
+    }
+    CU(h, cudaGetLastError());
+    return OOKD_OK;
+}
+
+int ookd_gpu_levels(ookd_gpu *h, const int16_t *iq, int iq_is_device_ptr, uint64_t first_sample, uint64_t n_samples,
+                    uint64_t *hist)
+{
+    if (!h || !hist) return OOKD_ERR_ARG;
+    if (!iq && n_samples) return fail(h, OOKD_ERR_ARG, "levels: null input");
+    const u64 D = h->total_dec;
+    if (first_sample % D) return fail(h, OOKD_ERR_ARG, "levels: first_sample must be a multiple of the total decimation");
+    memset(hist, 0, OOKD_LEVEL_BINS * sizeof(uint64_t));
+    const i64 o_lo = (i64) (first_sample / D), o_hi = (i64) ((first_sample + n_samples) / D);
+    if (o_hi <= o_lo) return OOKD_OK;
+    CU(h, cudaSetDevice(h->device));
+    const u64 halo_avail = first_sample < h->halo ? first_sample : h->halo;
+    const i64 in_base = (i64) (first_sample - halo_avail), in_valid_end = (i64) (first_sample + n_samples);
+    DevBuf tmp_in, d_hist, staged;
+    const void *d_in = nullptr;
+    int rc = stage_input(h, iq, iq_is_device_ptr != 0, (halo_avail + n_samples) * h->in_bytes, tmp_in, &d_in);
+    if (!rc) rc = ensure(h, d_hist, OOKD_LEVEL_BINS * sizeof(u64));
+    if (!rc && cudaMemsetAsync(d_hist.p, 0, OOKD_LEVEL_BINS * sizeof(u64), h->s_compute) != cudaSuccess) {
+        rc = fail(h, OOKD_ERR_CUDA, "levels: memset failed");
+    }
+    if (!rc && h->stages.size() == 1) {
+        rc = launch_levels(h, d_in, true, in_base, in_valid_end, o_lo, o_hi, (u64 *) d_hist.p);
+    } else if (!rc) {
+        // stages 1..S-1 through the generic chain into a bounded staging buffer (about 2^24 of their outputs per piece),
+        // then the last stage, power and bins from there
+        const Stage &last = h->stages.back();
+        const i64 piece = std::max<i64>(1, (i64) (1u << 24) / (i64) last.D);
+        for (i64 o = o_lo; !rc && o < o_hi; o += piece) {
+            const i64 e = std::min(o + piece, o_hi);
+            // last-stage output j reads stage S-1 outputs (j+1)*D-1-(T-1) .. (j+1)*D-1
+            const i64 lo = std::max<i64>(0, (o + 1) * (i64) last.D - (i64) last.T), hi = e * (i64) last.D;
+            rc = ensure(h, staged, (size_t) (hi - lo) * sizeof(float2));
+            if (!rc) rc = run_generic_chain(h, d_in, true, in_base, in_valid_end, lo, hi, (float2 *) staged.p, nullptr, 0,
+                                            h->stages.size() - 1);
+            if (!rc) rc = launch_levels(h, staged.p, false, lo, hi, o, e, (u64 *) d_hist.p);
+        }
+    }
+    if (!rc) {
+        cudaError_t e = cudaMemcpyAsync(hist, d_hist.p, OOKD_LEVEL_BINS * sizeof(u64), cudaMemcpyDeviceToHost, h->s_compute);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(h->s_compute);
+        if (e != cudaSuccess) rc = fail(h, OOKD_ERR_CUDA, "levels: %s", cudaGetErrorString(e));
+    }
+    cudaStreamSynchronize(h->s_compute);
+    release(tmp_in);
+    release(d_hist);
+    release(staged);
+    if (rc) memset(hist, 0, OOKD_LEVEL_BINS * sizeof(uint64_t));
     return rc;
 }
 

@@ -406,3 +406,49 @@ int ookd_tune_sc16q11(const int16_t *in, int16_t *out, uint64_t first_sample, ui
     }
     return OOKD_OK;
 }
+
+/*
+ * Levels (include/ookd_gpu.h, "Levels"): the threshold rule on a level histogram.  The median bin is found in integer
+ * arithmetic (cum >= n - cum cannot overflow where 2 cum >= n could), and the floor is the upper edge of that bin, a
+ * float read off its bits, so the result is a stated function of the counts.
+ */
+int ookd_level_threshold(const uint64_t *hist, double margin_db, float *threshold, double *floor_power)
+{
+    if (!hist || !threshold || !isfinite(margin_db)) {
+        return OOKD_ERR_ARG;
+    }
+    uint64_t n = 0;
+    for (int b = 0; b < OOKD_LEVEL_BINS; b++) {
+        if (hist[b] > UINT64_MAX - n) {
+            return OOKD_ERR_ARG;                /* more outputs than a uint64 counts */
+        }
+        n += hist[b];
+    }
+    if (n == 0) {
+        return OOKD_ERR_ARG;
+    }
+    uint64_t cum = 0;
+    uint32_t m = 0;
+    for (;; m++) {
+        cum += hist[m];
+        if (cum >= n - cum) {
+            break;
+        }
+    }
+    if (m >= 4079) {
+        return OOKD_ERR_ARG;                    /* the upper edge 4080 << 19 is +inf, and the bins above are NaN */
+    }
+    const uint32_t edge = (m + 1) << 19;
+    float f;
+    memcpy(&f, &edge, sizeof(f));
+    const double F = (double) f;
+    const float thr = (float) sqrt(F * pow(10.0, margin_db / 10.0));
+    if (!isfinite(thr)) {
+        return OOKD_ERR_ARG;
+    }
+    *threshold = thr;
+    if (floor_power) {
+        *floor_power = F;
+    }
+    return OOKD_OK;
+}

@@ -80,6 +80,9 @@ static void usage(const char *argv0)
     printf("  -p, --tx-param <name=value>   Device parameter value to transmit.\n\n");
     printf("Receive options:\n");
     printf("  -T, --rx-threshold <value>    On/Off threshold. Range is 0.0 to 1.0. Default: 0.1\n");
+    printf("  -T auto[:<dB>]                Choose the threshold from the first window's noise floor: <dB> (signed,\n");
+    printf("                                default 12) above its median filtered power.  Printed on stderr, so\n");
+    printf("                                that passing it back as -T <value> decodes the same.\n");
     printf("  -F, --rx-filter <filename>    Filter name or path; \"none\" disables filtering.\n");
     printf("  -R, --rx-rec <[type,]file>    Record the filtered samples (SC16Q11) to a file.\n");
     printf("  --rx-rec-input                Record the input samples instead of the filtered ones.\n");
@@ -137,6 +140,25 @@ static bool parse_offset(const char *s, double *out)
     else if (*end != '\0') return false;
     *out = v * mult;
     return isfinite(*out);
+}
+
+/* -T auto, -T auto:<dB>: a signed decimal margin over the median power */
+static bool parse_auto_threshold(const char *s, double *margin_db)
+{
+    if (!strcmp(s, "auto")) {
+        *margin_db = OOKD_LEVEL_MARGIN_DB;
+        return true;
+    }
+    if (strncmp(s, "auto:", 5) || !s[5]) {
+        return false;
+    }
+    char *end;
+    const double v = strtod(s + 5, &end);
+    if (end == s + 5 || *end || !isfinite(v)) {
+        return false;
+    }
+    *margin_db = v;
+    return true;
 }
 
 static bool parse_level(const char *s, enum ookd_log_level *out)
@@ -209,6 +231,16 @@ int main(int argc, char *argv[])
                 break;
             }
             case 'T': {
+                if (!strncmp(optarg, "auto", 4)) {
+                    if (!parse_auto_threshold(optarg, &cfg.rx_threshold_margin_db)) {
+                        fprintf(stderr, "Invalid RX threshold: %s (automatic forms: \"auto\" or \"auto:<dB>\", a signed "
+                                "margin in dB over the median power)\n", optarg);
+                        return EXIT_FAILURE;
+                    }
+                    cfg.rx_threshold_auto = true;
+                    break;
+                }
+                cfg.rx_threshold_auto = false;
                 const double v = strtod(optarg, &end);
                 if (end == optarg || *end || v < 0.0 || v > 1.0) {
                     fprintf(stderr, "Invalid RX threshold: %s\n", optarg);
@@ -361,6 +393,10 @@ int main(int argc, char *argv[])
         }
         if (offset_arg) {
             fprintf(stderr, "Error: --rx-offset cannot be used with --tx.\n");
+            return EXIT_FAILURE;
+        }
+        if (cfg.rx_threshold_auto) {
+            fprintf(stderr, "Error: -T auto cannot be used with --tx.\n");
             return EXIT_FAILURE;
         }
         status = ookd_tx(&cfg);

@@ -109,6 +109,9 @@ struct ookd_cfg {                       /* the fields of struct ookiedokie_cfg t
     uint64_t window_samples;            /* samples per decode window, 0 => default (2^26 per GPU)             */
     enum ookd_rx_fmt rx_fmt;
     float    rx_threshold;
+    bool     rx_threshold_auto;         /* -T auto[:<dB>]: rx_threshold is chosen from the first window's level histogram
+                                           (ookd_gpu_levels, ookd_level_threshold) before any window is decoded   */
+    double   rx_threshold_margin_db;    /* ... its margin over the median power, in dB                              */
     unsigned int samplerate;
     unsigned int samples_per_buffer;
     unsigned int tx_count;

@@ -10,6 +10,7 @@
 #define _GNU_SOURCE
 #include "ookd_host.h"
 
+#include <assert.h>
 #include <errno.h>
 #include <inttypes.h>
 #include <pthread.h>
@@ -305,6 +306,59 @@ static int write_rec_input(struct rx_out *o, const struct rx_slot *s, uint64_t h
     return OOKD_OK;
 }
 
+/* The decode handles: one window over n_gpus > 1 GPUs (ids), or two handles used alternately on one GPU. */
+static int create_handles(const struct ookd_gpu_config *gc, unsigned n_gpus, const int32_t *ids, ookd_gpu *gpu[2],
+                          ookd_gpu_multi **multi)
+{
+    int rc;
+    if (n_gpus > 1) {
+        rc = ookd_gpu_multi_create(multi, gc, ids, n_gpus);
+        if (rc != OOKD_OK) {
+            log_error("Failed to set up the GPU receive path on %u GPUs: %s\n", n_gpus, ookd_gpu_strerror(rc));
+        }
+        return rc;
+    }
+    for (int i = 0; i < 2; i++) {
+        rc = ookd_gpu_create(&gpu[i], gc);
+        if (rc != OOKD_OK) {
+            log_error("Failed to set up the GPU receive path: %s\n", ookd_gpu_strerror(rc));
+            return rc;
+        }
+    }
+    return OOKD_OK;
+}
+
+/* -T auto: the threshold from the level histogram of the first window (samples [0, have) at p), by the rule of
+ * ookd_level_threshold.  h is the handle the histogram is taken on. */
+static int auto_threshold(ookd_gpu *h, const int16_t *p, uint64_t have, double margin_db, float *thr)
+{
+    uint64_t *hist = calloc(OOKD_LEVEL_BINS, sizeof(uint64_t));
+    if (!hist) {
+        return OOKD_ERR_NOMEM;
+    }
+    int rc = ookd_gpu_levels(h, p, 0, 0, have, hist);
+    if (rc != OOKD_OK) {
+        log_error("Level histogram failed: %s (%s)\n", ookd_gpu_strerror(rc), ookd_gpu_last_error(h));
+        free(hist);
+        return rc;
+    }
+    uint64_t n = 0;
+    for (int b = 0; b < OOKD_LEVEL_BINS; b++) {
+        n += hist[b];
+    }
+    double floor_power = 0.0;
+    rc = ookd_level_threshold(hist, margin_db, thr, &floor_power);
+    free(hist);
+    if (rc != OOKD_OK) {
+        log_error("No automatic threshold: the first window's %" PRIu64 " filtered outputs have no finite median power "
+                  "or the margin of %g dB gives no finite threshold; pass -T <value>.\n", n, margin_db);
+        return rc;
+    }
+    ookd_log(OOKD_LOG_INFO, "Auto threshold: median power %.9g over %" PRIu64 " outputs, margin %g dB -> threshold %.9g\n",
+             floor_power, n, margin_db, (double) *thr);
+    return OOKD_OK;
+}
+
 int ookd_rx(const struct ookd_cfg *cfg)
 {
     int status = -1;
@@ -378,36 +432,24 @@ int ookd_rx(const struct ookd_cfg *cfg)
     gc.tune_step = cfg->tune_step;
     const unsigned n_gpus = cfg->n_gpus > 1 ? cfg->n_gpus : 1;
     int rc;
-    uint32_t halo;
-    if (n_gpus > 1) {
-        /* one window over several GPUs: time shards with FIR halos, carries stitched on the host */
-        int32_t ids[64];
-        if (n_gpus > 64) {
-            log_error("At most 64 GPUs.\n");
-            goto out;
-        }
-        for (unsigned g = 0; g < n_gpus; g++) {
-            ids[g] = cfg->gpu_ids ? cfg->gpu_ids[g] : (cfg->gpu_id > 0 ? cfg->gpu_id : 0) + (int32_t) g;
-        }
-        rc = ookd_gpu_multi_create(&multi, &gc, ids, n_gpus);
-        if (rc != OOKD_OK) {
-            log_error("Failed to set up the GPU receive path on %u GPUs: %s\n", n_gpus, ookd_gpu_strerror(rc));
-            goto out;
-        }
-        halo = ookd_gpu_multi_halo(multi);
-    } else {
-        /* two handles used alternately: window w+1 is enqueued (H2D + screening) before window w is waited for, entered
-         * from one chunk of warm-up history and corrected afterwards if its predecessor's exit says otherwise */
-        gc.sm_warmup = gc.sm ? 1 : 0;
-        for (int i = 0; i < 2; i++) {
-            rc = ookd_gpu_create(&gpu[i], &gc);
-            if (rc != OOKD_OK) {
-                log_error("Failed to set up the GPU receive path: %s\n", ookd_gpu_strerror(rc));
-                goto out;
-            }
-        }
-        halo = ookd_gpu_halo(gpu[0]);
+    /* n_gpus > 1: one window over several GPUs, time shards with FIR halos, carries stitched on the host.  One GPU: two
+     * handles used alternately: window w+1 is enqueued (H2D + screening) before window w is waited for, entered from
+     * one chunk of warm-up history and corrected afterwards if its predecessor's exit says otherwise. */
+    int32_t ids[64];
+    if (n_gpus > 64) {
+        log_error("At most 64 GPUs.\n");
+        goto out;
     }
+    for (unsigned g = 0; g < n_gpus; g++) {
+        ids[g] = cfg->gpu_ids ? cfg->gpu_ids[g] : (cfg->gpu_id > 0 ? cfg->gpu_id : 0) + (int32_t) g;
+    }
+    if (n_gpus == 1) {
+        gc.sm_warmup = gc.sm ? 1 : 0;
+    }
+    if (create_handles(&gc, n_gpus, ids, gpu, &multi) != OOKD_OK) {
+        goto out;
+    }
+    const uint32_t halo = multi ? ookd_gpu_multi_halo(multi) : ookd_gpu_halo(gpu[0]);
 
     /* window = whole buffers, aligned for sharding */
     const uint64_t spb = cfg->samples_per_buffer;
@@ -448,6 +490,25 @@ int ookd_rx(const struct ookd_cfg *cfg)
     struct ookd_sm_carry prev_exit;
     memset(&prev_exit, 0, sizeof(prev_exit));
     struct rx_slot *cur = reader_wait(&rd, 0);
+    if (cfg->rx_threshold_auto && cur->have > 0) {
+        /* the threshold is fixed for the whole run: chosen from the first window, then the decode handles are created
+         * with it (no entry point changes a live handle's threshold) */
+        const int16_t *p0 = (const int16_t *) (cur->buf + rd.bps * (size_t) halo);
+        if (auto_threshold(multi ? ookd_gpu_multi_handle(multi, 0) : gpu[0], p0, cur->have, cfg->rx_threshold_margin_db,
+                           &gc.threshold) != OOKD_OK) {
+            goto out;
+        }
+        ookd_gpu_destroy(gpu[0]);
+        ookd_gpu_destroy(gpu[1]);
+        ookd_gpu_multi_destroy(multi);
+        gpu[0] = gpu[1] = NULL;
+        multi = NULL;
+        if (create_handles(&gc, n_gpus, ids, gpu, &multi) != OOKD_OK) {
+            goto out;
+        }
+        /* the windows and their history were laid out for this halo, and it does not depend on the threshold */
+        assert((multi ? ookd_gpu_multi_halo(multi) : ookd_gpu_halo(gpu[0])) == halo);
+    }
     bool begun = false;                                     /* window w already enqueued on gpu[w % 2] */
     for (unsigned w = 0;; w++) {
         struct ookd_gpu_result res;
