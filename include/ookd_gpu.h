@@ -192,6 +192,28 @@ int ookd_tune_sc16q11(const int16_t *in, int16_t *out, uint64_t first_sample, ui
 #define OOKD_LEVEL_MARGIN_DB  12.0
 int ookd_level_threshold(const uint64_t *hist, double margin_db, float *threshold, double *floor_power);
 
+/* ---- Deglitch: remove short runs from the on/off decisions before anything consumes them ----
+ * Let r(i) be the threshold decision of global output i (post-decimation), with r(i) = 0 for i < 0.  With
+ * ookd_gpu_config.deglitch = M >= 1 the decision stream becomes the majority of the last 2M+1 decisions,
+ *
+ *     v(i) = [ r(i-2M) + ... + r(i-1) + r(i)  >=  M + 1 ],
+ *
+ * and every consumer of decisions sees v instead of r: the edge list and first_bit (ookd_gpu_edges, --rx-rec-dig),
+ * ookd_gpu_bits, and the state machine, so messages, out_sample and buffer_idx.  The filtered samples
+ * (ookd_gpu_filtered, _filtered_sc16q11), ookd_gpu_levels and the input are unchanged.  Consequences:
+ *   - an isolated run of at most M outputs disappears;
+ *   - a run of at least M+1 outputs between long opposite runs keeps its exact length;
+ *   - every edge of a clean signal is delayed by exactly M outputs;
+ *   - v(0) = 0;
+ *   - a transmission that ends within M outputs of the capture's end may be cut.
+ * v(i) depends on a bounded history of r, as a filtered output depends on a bounded history of input, so shards,
+ * sub-windows, multi-GPU splits and windows of the CLI need no new state: ookd_gpu_halo() grows by
+ * roundup(2M, 64) * total decimation input samples, and callers that size their history from it need nothing else.
+ * The vote is causal on purpose: a centred one would need future input at the end of every non-final shard.
+ * M = 0: off, the decode runs exactly as without this field.  M > OOKD_DEGLITCH_MAX, or a halo that no longer fits
+ * in 32 bits, is OOKD_ERR_ARG from ookd_gpu_create (checked before any CUDA call). */
+#define OOKD_DEGLITCH_MAX     65535u
+
 /* ---- results ---- */
 struct ookd_msg {
     uint64_t out_sample;                     /* post-decimation index of the sample that
@@ -242,6 +264,8 @@ struct ookd_gpu_config {
                                                 after a decode that was cut (OOKD_ERR_STATE).  Implies sm_warmup.  0, 1: off */
     uint32_t tune_step;                      /* != 0: decode the capture shifted down by a frequency offset (see
                                                 "Tuning" below; ookd_tune_step converts Hz).  0: off, today's kernels */
+    uint32_t deglitch;                       /* M >= 1: decisions are the majority of the last 2M+1 (see "Deglitch"
+                                                above); 0: off                                                        */
 };
 
 #define OOKD_FLAG_FORCE_GENERIC  1u          /* always use the shape-agnostic FIR kernels       */
@@ -426,7 +450,7 @@ void ookd_gpu_initial_carry(const ookd_gpu *h, struct ookd_sm_carry *c);  /* RES
  * with bit[i] != bit[i-1]; polarity alternates starting from !first_bit. */
 int  ookd_gpu_edges(ookd_gpu *h, const uint64_t **edges, uint64_t *n_edges, uint32_t *first_bit);
 
-/* Threshold decisions of the last decode, one byte per output sample. */
+/* Threshold decisions of the last decode, one byte per output sample (the voted ones with deglitch, see above). */
 int  ookd_gpu_bits(ookd_gpu *h, uint8_t *bits_out, uint64_t max_out, uint64_t *n_out);
 
 /* Filtered + decimated samples (interleaved float re,im) computed with the

@@ -19,6 +19,7 @@ MSG_BYTES = 32
 K_INF = 0xFFFFFFFF
 LEVEL_BINS = 4096
 LEVEL_MARGIN_DB = 12.0
+DEGLITCH_MAX = 65535
 
 FLAG_FORCE_GENERIC = 1
 FLAG_NO_SCREEN = 2
@@ -128,10 +129,21 @@ class SmCarry(C.Structure):
 
 
 class GpuConfig(C.Structure):
+    """struct ookd_gpu_config up to tune_step, the layout of earlier releases.  The whole struct is GpuConfigEx below:
+    use it for new code (Gpu and MultiGpu do)."""
     _fields_ = [("filter", C.POINTER(FilterDesc)), ("sm", C.POINTER(SmDesc)), ("threshold", C.c_float),
                 ("samples_per_buffer", C.c_uint32), ("device_id", C.c_int32), ("flags", C.c_uint32),
                 ("sm_chunk_buffers", C.c_uint32), ("sm_warmup", C.c_uint32), ("sm_burst_rounds", C.c_uint32),
                 ("sub_windows", C.c_uint32), ("tune_step", C.c_uint32)]
+
+
+class GpuConfigEx(C.Structure):
+    """struct ookd_gpu_config with every field.  GpuConfig ends at tune_step: the appended deglitch lies in its tail
+    padding (both are 56 bytes), which ctypes zero-fills, so a GpuConfig still describes a handle with deglitch = 0."""
+    _fields_ = GpuConfig._fields_ + [("deglitch", C.c_uint32)]
+
+
+assert C.sizeof(GpuConfigEx) == C.sizeof(GpuConfig)
 
 
 class GpuResult(C.Structure):
@@ -181,7 +193,7 @@ def lib():
         L.ookd_gpu_last_error.restype = C.c_char_p
         L.ookd_gpu_last_error.argtypes = [C.c_void_p]
         L.ookd_gpu_create.restype = C.c_int
-        L.ookd_gpu_create.argtypes = [C.POINTER(C.c_void_p), C.POINTER(GpuConfig)]
+        L.ookd_gpu_create.argtypes = [C.POINTER(C.c_void_p), C.c_void_p]              # GpuConfig or GpuConfigEx
         L.ookd_gpu_destroy.argtypes = [C.c_void_p]
         L.ookd_gpu_decode.restype = C.c_int
         L.ookd_gpu_decode.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.POINTER(GpuResult)]
@@ -225,7 +237,7 @@ def lib():
         L.ookd_gpu_filtered_sc16q11.restype = C.c_int
         L.ookd_gpu_filtered_sc16q11.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
         L.ookd_gpu_multi_create.restype = C.c_int
-        L.ookd_gpu_multi_create.argtypes = [C.POINTER(C.c_void_p), C.POINTER(GpuConfig), C.POINTER(C.c_int32), C.c_uint32]
+        L.ookd_gpu_multi_create.argtypes = [C.POINTER(C.c_void_p), C.c_void_p, C.POINTER(C.c_int32), C.c_uint32]
         L.ookd_gpu_multi_destroy.argtypes = [C.c_void_p]
         L.ookd_gpu_multi_halo.restype = C.c_uint32
         L.ookd_gpu_multi_halo.argtypes = [C.c_void_p]
@@ -421,15 +433,17 @@ class Gpu:
     """One ookd_gpu handle.  input_format: "sc16q11" (int16 I,Q), "cs8" (int8 I,Q) or "cu8" (uint8 I,Q) host arrays;
     an 8-bit capture decodes exactly as its widened SC16Q11 capture does (include/ookd_gpu.h, OOKD_FLAG_INPUT_*).
     tune_step != 0 (see tune_step()): decode the capture shifted down by that frequency offset, exactly as the untuned
-    handle decodes the rotated capture T(x) (include/ookd_gpu.h, "Tuning")."""
+    handle decodes the rotated capture T(x) (include/ookd_gpu.h, "Tuning").
+    deglitch = M >= 1: every consumer of decisions sees the majority of the last 2M+1 (include/ookd_gpu.h,
+    "Deglitch"); M > DEGLITCH_MAX is an OokdError from ookd_gpu_create."""
 
     def __init__(self, filter_stages=None, sm=None, threshold=0.1, samples_per_buffer=8192, device_id=-1,
                  flags=0, sm_chunk_buffers=0, sm_warmup=0, sm_burst_rounds=0, sub_windows=0, input_format="sc16q11",
-                 tune_step=0):
+                 tune_step=0, deglitch=0):
         flags |= _input_format(input_format, flags)[0]
         self.input_format = input_format
         L = lib()
-        cfg = GpuConfig()
+        cfg = GpuConfigEx()
         self._keep = []
         if filter_stages:
             fd, k = make_filter_desc(filter_stages)
@@ -451,6 +465,7 @@ class Gpu:
         cfg.sm_burst_rounds = sm_burst_rounds
         cfg.sub_windows = sub_windows
         cfg.tune_step = tune_step
+        cfg.deglitch = deglitch
         self.h = C.c_void_p()
         rc = L.ookd_gpu_create(C.byref(self.h), C.byref(cfg))
         if rc != 0:
@@ -605,11 +620,11 @@ class MultiGpu:
     """One ookd_gpu_multi handle: a window time-sharded over several GPUs of this process."""
 
     def __init__(self, gpu_ids, filter_stages=None, sm=None, threshold=0.1, samples_per_buffer=8192, flags=0,
-                 sm_chunk_buffers=0, input_format="sc16q11", tune_step=0):
+                 sm_chunk_buffers=0, input_format="sc16q11", tune_step=0, deglitch=0):
         flags |= _input_format(input_format, flags)[0]
         self.input_format = input_format
         L = lib()
-        cfg = GpuConfig()
+        cfg = GpuConfigEx()
         self._keep = []
         if filter_stages:
             fd, k = make_filter_desc(filter_stages)
@@ -627,6 +642,7 @@ class MultiGpu:
         cfg.flags = flags
         cfg.sm_chunk_buffers = sm_chunk_buffers
         cfg.tune_step = tune_step
+        cfg.deglitch = deglitch
         ids = (C.c_int32 * len(gpu_ids))(*gpu_ids)
         self.h = C.c_void_p()
         rc = L.ookd_gpu_multi_create(C.byref(self.h), C.byref(cfg), ids, len(gpu_ids))

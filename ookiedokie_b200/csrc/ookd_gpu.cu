@@ -25,6 +25,7 @@
 #include "sm_kernels.cuh"
 #include "synth_kernel.cuh"
 #include "level_kernels.cuh"
+#include "vote_kernels.cuh"
 
 using namespace ookd;
 
@@ -87,6 +88,8 @@ struct ookd_gpu {
     int fmt = FMT_SC16Q11;            // capture format (OOKD_FLAG_INPUT_*, input_fmt.cuh), + FMT_TUNED with a tune step
     uint32_t in_bytes = 4;            // ... its bytes per sample
     uint32_t tune_step = 0;           // cfg.tune_step (ookd_gpu.h, "Tuning"); kernels ignore it unless fmt is tuned
+    uint32_t deglitch = 0;            // cfg.deglitch = M (ookd_gpu.h, "Deglitch"); 0: the FIR writes `bits` directly
+    uint32_t vote_r = 0;              // roundup(2M, 64): outputs of raw decisions the vote reads in front of bit_base
     bool screen = false;
     bool screen2 = false;             // dec4 shape: screen + refine (else the exact tiled two-stage kernel)
     bool fma = false;                 // FMA screening (fused multiply-add pass + rigorous band, exact refine of the band):
@@ -104,7 +107,7 @@ struct ookd_gpu {
     SmTable *d_tab = nullptr;
 
     // workspaces
-    DevBuf in, bits, inter[2], block_counts, edges, scalars, chunk_exit[2], chunk_ran, slots, slot_count,
+    DevBuf in, bits, raw_bits, inter[2], block_counts, edges, scalars, chunk_exit[2], chunk_ran, slots, slot_count,
            sm_dbg, slot_off, msgs_dev, dense_list, chunk_e, bound_pos, seed_pos, seed_e, seed_kind, edge_tmp, final_entry, tab_entry, tab_exit, tab_nmsg, tab_cnt[2], tab_link, tab_chosen;
     uint32_t slot_cap = 8;
     bool tables_valid = false;       // entry/exit tables of the last decode can be extended by resolve
@@ -129,6 +132,8 @@ struct ookd_gpu {
     // geometry of the last decode (needed by resolve / edges / bits)
     bool have_last = false;
     i64 out_lo = 0, out_hi = 0, bit_base = 0;
+    i64 fir_base = 0;                 // first output the FIR / threshold stage decides: bit_base, or with deglitch
+                                      // max(0, bit_base - vote_r) (its decisions then go to raw_bits)
     uint32_t pre = 0;
     u64 n_edges = 0, first_buffer = 0, n_buffers = 0, n_in = 0;
     uint32_t n_chunks = 0, base_bit = 0;
@@ -401,12 +406,18 @@ cudaEvent_t *screen_token(int device)
     return &tokens[device];
 }
 
+// Where the FIR / threshold stage writes its decisions: the consumers' array, or with deglitch the vote's input.
+uint32_t *fir_bits(ookd_gpu *h)
+{
+    return (uint32_t *) (h->deglitch ? h->raw_bits.p : h->bits.p);
+}
+
 TiledArgs tiled_args(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_valid_end)
 {
     TiledArgs a{};
     a.in = d_in; a.in_base = in_base; a.in_valid_end = in_valid_end;
-    a.out_lo = h->bit_base; a.out_hi = h->out_hi;
-    a.out_bits = (uint8_t *) h->bits.p; a.bit_base = h->bit_base; a.pstar = h->pstar;
+    a.out_lo = h->fir_base; a.out_hi = h->out_hi;
+    a.out_bits = (uint8_t *) fir_bits(h); a.bit_base = h->fir_base; a.pstar = h->pstar;
     return a;
 }
 
@@ -425,7 +436,7 @@ ScreenArgs screen_args(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_va
 #endif
 
 // TMA-staged screening kernel (screen_tma.cuh) over `tiles` tiles of 4096 INPUT samples starting at tile
-// sa.tile_offset (tiles are numbered from h->bit_base in units of 4096 / dec outputs).
+// sa.tile_offset (tiles are numbered from h->fir_base in units of 4096 / dec outputs).
 int launch_screen_tma(ookd_gpu *h, const ScreenArgs &sa, const ScreenParams &sp, const uint32_t *d_in, i64 in_base,
                       i64 in_valid_end, u64 tiles, int dec)
 {
@@ -436,7 +447,7 @@ int launch_screen_tma(ookd_gpu *h, const ScreenArgs &sa, const ScreenParams &sp,
     ta.s = sa;
     const i64 rs = 128 / h->in_bytes;                         // samples per row
     const i64 first_present = in_base > 0 ? in_base : 0;
-    i64 row0 = h->bit_base * dec;
+    i64 row0 = h->fir_base * dec;
     if (row0 < first_present) row0 += (first_present - row0 + STMA_L - 1) / STMA_L * STMA_L;
     const uintptr_t addr0 = (uintptr_t) d_in + (uintptr_t) ((row0 - in_base) * h->in_bytes);
     const i64 n_rows = (in_valid_end - row0) / rs;
@@ -456,8 +467,8 @@ int launch_screen_tma(ookd_gpu *h, const ScreenArgs &sa, const ScreenParams &sp,
     }
     ta.row0_sample = row0;
     if (ok) {
-        ta.fast_lo = (uint32_t) ((row0 - h->bit_base * dec) / STMA_L);
-        ta.fast_hi = (uint32_t) ((row0 + n_rows * rs - h->bit_base * dec) / STMA_L);
+        ta.fast_lo = (uint32_t) ((row0 - h->fir_base * dec) / STMA_L);
+        ta.fast_hi = (uint32_t) ((row0 + n_rows * rs - h->fir_base * dec) / STMA_L);
     } else {
         ta.fast_lo = ta.fast_hi = 0;
     }
@@ -485,7 +496,7 @@ int launch_fir(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_valid_end,
         const u64 tiles = (u64) (o_end - o_begin + TILE_L - 1) / TILE_L;
         if (h->screen) {
             const u64 stiles = (u64) (o_end - o_begin + SCREEN_L - 1) / SCREEN_L;
-            const u64 tile0 = (u64) (o_begin - h->bit_base) / SCREEN_L;
+            const u64 tile0 = (u64) (o_begin - h->fir_base) / SCREEN_L;
             ScreenArgs sa = screen_args(h, d_in, in_base, in_valid_end);
             sa.t.out_hi = o_end;
             sa.tile_offset = (uint32_t) tile0;
@@ -521,7 +532,7 @@ int launch_fir(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_valid_end,
         const u64 tiles = (u64) (o_end - o_begin + L2 - 1) / L2;
         ScreenArgs sa = screen_args(h, d_in, in_base, in_valid_end);
         sa.t.out_hi = o_end;
-        sa.tile_offset = (uint32_t) ((u64) (o_begin - h->bit_base) / L2);
+        sa.tile_offset = (uint32_t) ((u64) (o_begin - h->fir_base) / L2);
         sa.n_tiles = (uint32_t) tiles;
         ScreenParams sp;
         make_screen_params_dec4(h, sp);
@@ -562,7 +573,7 @@ int launch_fir(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_valid_end,
 int launch_fir_refine(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_valid_end)
 {
     if (h->path == FIR_SCREEN_DEC4 && !(h->screen2 || h->fma)) return OOKD_OK;
-    if (h->path == FIR_SCREEN_DEC4 && h->out_hi > h->bit_base) {
+    if (h->path == FIR_SCREEN_DEC4 && h->out_hi > h->fir_base) {
         Taps2Param tp;
         memcpy(tp.t1, h->stages[0].taps.data(), sizeof(tp.t1));
         memcpy(tp.t2, h->stages[1].taps.data(), sizeof(tp.t2));
@@ -576,7 +587,7 @@ int launch_fir_refine(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_val
         CU(h, cudaGetLastError());
         return OOKD_OK;
     }
-    if (!(h->path == FIR_TILED_1STAGE_32 && (h->screen || h->fma)) || h->out_hi <= h->bit_base) return OOKD_OK;
+    if (!(h->path == FIR_TILED_1STAGE_32 && (h->screen || h->fma)) || h->out_hi <= h->fir_base) return OOKD_OK;
     TapsParam<32> tp;
     memcpy(tp.t, h->stages[0].taps.data(), sizeof(tp.t));
     ScreenArgs sa = screen_args(h, d_in, in_base, in_valid_end);
@@ -599,7 +610,28 @@ int launch_fir_exact_all(ookd_gpu *h, const uint32_t *d_in, i64 in_base, i64 in_
     h->adaptive = false;
     h->adaptive_ok = false;
     h->fma = false;
-    return launch_fir(h, d_in, in_base, in_valid_end, h->bit_base, h->out_hi);
+    return launch_fir(h, d_in, in_base, in_valid_end, h->fir_base, h->out_hi);
+}
+
+// Deglitch: the voted decisions of [bit_base, out_hi) from the raw ones of [fir_base, out_hi).  Nothing without it.
+int launch_vote(ookd_gpu *h)
+{
+    if (!h->deglitch || h->out_hi <= h->bit_base) return OOKD_OK;
+    VoteArgs a{};
+    a.raw = (const u64 *) h->raw_bits.p;
+    a.voted = (u64 *) h->bits.p;
+    a.off = h->bit_base - h->fir_base;
+    a.n_raw = h->out_hi - h->fir_base;
+    a.n_words = (h->out_hi - h->bit_base + 63) / 64;
+    a.m = h->deglitch;
+    // a warp's first window costs R / 2048 loads per lane: a stretch of at least twice that many rounds of 32 words
+    // keeps it below the sliding work
+    a.wpw = 32 * std::max<uint32_t>(8, 2 * ((h->vote_r + 2047) / 2048));
+    const u64 warps = ((u64) a.n_words + a.wpw - 1) / a.wpw;
+    vote_kernel<<<(unsigned) ((warps + VOTE_NT / 32 - 1) / (VOTE_NT / 32)), VOTE_NT, 0, h->s_compute>>>(a);
+    h->launches++;
+    CU(h, cudaGetLastError());
+    return OOKD_OK;
 }
 
 // ---- shape-agnostic chain: one launch per stage, intermediates in HBM ----
@@ -1460,6 +1492,22 @@ int decode_tail_fast_finish(ookd_gpu *h, ookd_sm_carry *exit_, ookd_gpu_result *
     return finish_messages(h, h->h_msgs_pin, n_msgs, last, rounds, exit_, res);
 }
 
+// The halo of a deglitch handle, H + (8 + roundup(2M, 64)) * D rounded up to 16 bytes of input, fits in 32 bits: decided
+// from the configuration alone, so that ookd_gpu_create rejects it before any CUDA call.  (A malformed filter is
+// rejected later, with the same status.)
+bool deglitch_halo_fits(const ookd_gpu_config *cfg)
+{
+    u64 dec = 1, halo = 0;
+    const ookd_filter_desc *f = cfg->filter;
+    for (uint32_t s = 0; f && s < f->num_stages && s < OOKD_MAX_STAGES; s++) {
+        if (f->num_taps[s] > 0) halo += (u64) (f->num_taps[s] - 1) * dec;
+        dec *= f->decimation[s] ? f->decimation[s] : 1;
+        if (dec > 0xFFFFFFFFull) return true;                          // (rejected with the filter)
+    }
+    const u64 vote_r = (2 * (u64) cfg->deglitch + 63) & ~63ull;
+    return halo + (8 + vote_r) * dec + 15 <= 0xFFFFFFFFull;
+}
+
 }  // namespace
 
 // =======================================================================================
@@ -1502,7 +1550,7 @@ void ookd_gpu_destroy(ookd_gpu *h)
     h->tail_graph = nullptr;
     for (auto &st : h->stages) if (st.d_taps) cudaFree(st.d_taps);
     if (h->d_tab) cudaFree(h->d_tab);
-    DevBuf *all[] = {&h->in, &h->bits, &h->inter[0], &h->inter[1], &h->block_counts, &h->edges, &h->scalars,
+    DevBuf *all[] = {&h->in, &h->bits, &h->raw_bits, &h->inter[0], &h->inter[1], &h->block_counts, &h->edges, &h->scalars,
                      &h->chunk_exit[0], &h->chunk_exit[1], &h->chunk_ran, &h->slots, &h->slot_count,
                      &h->sm_dbg, &h->slot_off, &h->msgs_dev, &h->dense_list, &h->chunk_e, &h->bound_pos, &h->seed_pos, &h->seed_e, &h->seed_kind, &h->edge_tmp,
                      &h->final_entry, &h->tab_entry, &h->tab_exit, &h->tab_nmsg, &h->tab_cnt[0],
@@ -1527,6 +1575,8 @@ int ookd_gpu_create(ookd_gpu **out, const struct ookd_gpu_config *cfg)
     if (!out || !cfg || cfg->samples_per_buffer == 0) return OOKD_ERR_ARG;
     *out = nullptr;
     if ((cfg->flags & OOKD_FLAG_INPUT_CS8) && (cfg->flags & OOKD_FLAG_INPUT_CU8)) return OOKD_ERR_ARG;   // one format
+    if (cfg->deglitch > OOKD_DEGLITCH_MAX) return OOKD_ERR_ARG;
+    if (cfg->deglitch && !deglitch_halo_fits(cfg)) return OOKD_ERR_ARG;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return OOKD_ERR_CUDA;
     int dev = cfg->device_id;
@@ -1547,6 +1597,8 @@ int ookd_gpu_create(ookd_gpu **out, const struct ookd_gpu_config *cfg)
     h->fmt = (cfg->flags & OOKD_FLAG_INPUT_CS8) ? FMT_CS8 : (cfg->flags & OOKD_FLAG_INPUT_CU8) ? FMT_CU8 : FMT_SC16Q11;
     h->in_bytes = h->fmt == FMT_SC16Q11 ? 4 : 2;
     h->tune_step = cfg->tune_step;
+    h->deglitch = cfg->deglitch;
+    h->vote_r = (2 * cfg->deglitch + 63) & ~63u;
     if (h->tune_step) h->fmt |= FMT_TUNED;               // step 0: the untuned kernels, exactly
     h->chunk_buffers = cfg->sm_chunk_buffers ? cfg->sm_chunk_buffers : 64;
     h->warmup = cfg->sm_warmup != 0 || (cfg->sub_windows > 1 && cfg->sm);
@@ -1613,6 +1665,10 @@ int ookd_gpu_create(ookd_gpu **out, const struct ookd_gpu_config *cfg)
     // input (4 SC16Q11 samples, 8 8-bit samples) so that a shard pointer keeps the alignment the vector loads need
     const u64 halo_round = 16 / h->in_bytes - 1;
     h->halo = (uint32_t) ((halo + 8 * dec + halo_round) & ~halo_round);
+    if (h->deglitch) {
+        // the vote reads vote_r outputs of raw decisions in front of the first one it writes (fits: deglitch_halo_fits)
+        h->halo = (uint32_t) ((halo + (8 + (u64) h->vote_r) * dec + halo_round) & ~halo_round);
+    }
     if (h->warmup && cfg->sm) {
         // the warm-up history is exactly one chunk, and a chunk must be a whole number of lcm(spb, dec) units
         const u64 unit = dec / gcd64(h->spb, dec);
@@ -1768,26 +1824,31 @@ int ookd_gpu_decode_begin(ookd_gpu *h, const int16_t *iq, int iq_is_device_ptr, 
     h->out_hi = (i64) ((first_sample + n_eff) / D);
     h->pre = (h->out_lo > 0) ? 8 : 0;
     h->bit_base = h->out_lo - h->pre;
+    // (bit_base < 0 where a shard starts 1..7 outputs into the capture: the FIR kernels guard negative outputs, and the
+    // vote reads raw decisions before output 0 as 0)
+    h->fir_base = !h->deglitch ? h->bit_base : std::max<i64>(0, h->bit_base - (i64) h->vote_r);
     h->first_buffer = proc_first / spb;
     h->n_buffers = n_eff / spb;
     h->n_in = n_eff;
     const u64 n_bits = (u64) (h->out_hi - h->bit_base);
+    const u64 n_fir = (u64) (h->out_hi - h->fir_base);         // decisions the FIR / threshold stage takes (n_bits without deglitch)
     const u64 n_out = (u64) (h->out_hi - h->report_lo);
     h->n_chunks = (uint32_t) (((first_sample + n_eff - proc_first) / spb + h->chunk_buffers - 1) / h->chunk_buffers);
     if (h->n_chunks == 0) h->n_chunks = 1;
 
     int rc;
     if ((rc = ensure(h, h->bits, (n_bits / 8 + 64 + 8) & ~7ull))) return rc;
+    if (h->deglitch && (rc = ensure(h, h->raw_bits, (n_fir / 8 + 64 + 8) & ~7ull))) return rc;
 
     // Short captures (batches of independent ones, of unknown nature each): the probe kernel chooses the screening form
     // per decode.  Long ones: the probe and the wave of CTAs of the form not chosen would cost ~40 us per decode, so the
     // handle keeps its current form and switches once, for good, if the energy proofs overflow the work list.
-    h->adaptive = h->adaptive_ok && (h->screen || h->screen2) && !h->fma && n_bits <= (1ull << 26);
+    h->adaptive = h->adaptive_ok && (h->screen || h->screen2) && !h->fma && n_fir <= (1ull << 26);
     CU(h, cudaEventRecord(h->ev_t0, h->s_compute));
     if (h->screen || h->screen2 || h->fma) {
         // work list for undecided 8-output groups: room for 1/8 of all groups (beyond that the capture is
         // mostly "near the threshold" and screening is pointless)
-        const u64 groups = n_bits / 8 + 1;
+        const u64 groups = n_fir / 8 + 1;
         u64 cap = groups / 8 + 65536;
         if (cap > 0xFFFFFFF0ull) cap = 0xFFFFFFF0ull;
         h->work_cap = (uint32_t) cap;
@@ -1798,12 +1859,12 @@ int ookd_gpu_decode_begin(ookd_gpu *h, const int16_t *iq, int iq_is_device_ptr, 
     // ---- input staging + FIR/threshold ----
     const u64 n_have = halo_avail + n_samples;                 // samples present at iq
     auto launch_probe = [&](const uint32_t *d_src, i64 o_hi_probe) -> int {
-        if (!h->adaptive || o_hi_probe <= h->bit_base) return OOKD_OK;
+        if (!h->adaptive || o_hi_probe <= h->fir_base) return OOKD_OK;
         ScreenParams sp;
         if (h->path == FIR_SCREEN_DEC4) make_screen_params_dec4(h, sp); else make_screen_params(h, sp);
         TiledArgs pa{};
         pa.in = d_src; pa.in_base = in_base; pa.in_valid_end = in_valid_end;
-        pa.out_lo = h->bit_base; pa.out_hi = o_hi_probe;
+        pa.out_lo = h->fir_base; pa.out_hi = o_hi_probe;
         with_fmt(h->fmt, [&](auto fc) {
             screen_probe_kernel<decltype(fc)::value><<<1, 1024, 0, h->s_compute>>>(
                 pa, (int) h->total_dec, (int) h->halo_fir + 1, sp.k0, (uint32_t *) ((char *) h->scalars.p + 344), h->tune_step);
@@ -1827,7 +1888,7 @@ int ookd_gpu_decode_begin(ookd_gpu *h, const int16_t *iq, int iq_is_device_ptr, 
             CU(h, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
             h->ev_piece.push_back(e);
         }
-        i64 o_done = h->bit_base;
+        i64 o_done = h->fir_base;
         for (u64 p = 0; p < n_pieces; p++) {
             const u64 s0 = p * piece, s1 = (s0 + piece < n_have) ? s0 + piece : n_have;
             CU(h, cudaMemcpyAsync((char *) h->in.p + s0 * bps, (const char *) iq + s0 * bps, (s1 - s0) * bps,
@@ -1848,7 +1909,7 @@ int ookd_gpu_decode_begin(ookd_gpu *h, const int16_t *iq, int iq_is_device_ptr, 
                 } else {
                     const u64 g_end = (u64) in_base + s1;      // global samples present: [.., g_end)
                     o_avail = (i64) (g_end / D);
-                    o_avail = h->bit_base + (i64) (((u64) (o_avail - h->bit_base)) / TILE * TILE);
+                    o_avail = h->fir_base + (i64) (((u64) (o_avail - h->fir_base)) / TILE * TILE);
                     if (o_avail > h->out_hi) o_avail = h->out_hi;
                 }
                 if (o_avail > o_done) {
@@ -1859,25 +1920,26 @@ int ookd_gpu_decode_begin(ookd_gpu *h, const int16_t *iq, int iq_is_device_ptr, 
         }
         if (n_pieces == 0 && h->path != FIR_GENERIC) {
             if ((rc = launch_probe(d_in, h->out_hi))) return rc;
-            if ((rc = launch_fir(h, d_in, in_base, in_valid_end, h->bit_base, h->out_hi))) return rc;
+            if ((rc = launch_fir(h, d_in, in_base, in_valid_end, h->fir_base, h->out_hi))) return rc;
         }
         if (h->path == FIR_GENERIC) {
             if (n_pieces) CU(h, cudaStreamWaitEvent(h->s_compute, h->ev_piece[n_pieces - 1], 0));
-            if ((rc = run_generic_chain(h, d_in, true, in_base, in_valid_end, h->bit_base, h->out_hi, nullptr,
-                                        (uint32_t *) h->bits.p, h->bit_base))) return rc;
+            if ((rc = run_generic_chain(h, d_in, true, in_base, in_valid_end, h->fir_base, h->out_hi, nullptr,
+                                        fir_bits(h), h->fir_base))) return rc;
         }
     } else {
         if (h->path != FIR_GENERIC) {
             if ((rc = launch_probe(d_in, h->out_hi))) return rc;
-            if ((rc = launch_fir(h, d_in, in_base, in_valid_end, h->bit_base, h->out_hi))) return rc;
+            if ((rc = launch_fir(h, d_in, in_base, in_valid_end, h->fir_base, h->out_hi))) return rc;
         } else {
-            if ((rc = run_generic_chain(h, d_in, true, in_base, in_valid_end, h->bit_base, h->out_hi, nullptr,
-                                        (uint32_t *) h->bits.p, h->bit_base))) return rc;
+            if ((rc = run_generic_chain(h, d_in, true, in_base, in_valid_end, h->fir_base, h->out_hi, nullptr,
+                                        fir_bits(h), h->fir_base))) return rc;
         }
     }
     CU(h, cudaEventRecord(h->ev_s1, h->s_compute));
     if ((rc = launch_fir_refine(h, d_in, in_base, in_valid_end))) return rc;
     CU(h, cudaEventRecord(h->ev_f1, h->s_compute));
+    if ((rc = launch_vote(h))) return rc;
 
     // ---- edges + state machine: enqueued behind the FIR kernels when the single-synchronisation tail applies ----
     h->n_edges = 0;
@@ -1963,14 +2025,16 @@ static int decode_end_once(ookd_gpu *h, struct ookd_sm_carry *exit_, struct ookd
             h->adaptive_ok = false;
             h->fma = true;
             CU(h, cudaMemsetAsync((char *) h->scalars.p + 16, 0, 12, h->s_compute));
-            if ((rc = launch_fir(h, d_in, in_base, in_valid_end, h->bit_base, h->out_hi))) return rc;
+            if ((rc = launch_fir(h, d_in, in_base, in_valid_end, h->fir_base, h->out_hi))) return rc;
             if ((rc = launch_fir_refine(h, d_in, in_base, in_valid_end))) return rc;
+            if ((rc = launch_vote(h))) return rc;
             if ((rc = extract_edges(h, n_bits, res))) return rc;
             h->stat_dense_tiles = 1;
         }
         if ((h->screen || h->screen2 || h->fma) && h->stat_refined_blocks > h->work_cap) {
             // still too many (or no FMA form for this shape): decide everything exactly, and keep doing so
             if ((rc = launch_fir_exact_all(h, d_in, in_base, in_valid_end))) return rc;
+            if ((rc = launch_vote(h))) return rc;
             if ((rc = extract_edges(h, n_bits, res))) return rc;
             h->stat_dense_tiles = 1;
         }

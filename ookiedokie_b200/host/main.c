@@ -7,6 +7,8 @@
  * bladeRF hardware (frequency, bandwidth, gain, stream sizing) are accepted and ignored: a file's centre frequency is
  * fixed, and --rx-offset tunes to a transmitter away from it.
  */
+#include <ctype.h>
+#include <errno.h>
 #include <getopt.h>
 #include <limits.h>
 #include <math.h>
@@ -30,6 +32,7 @@
 #define OPT_WINDOW 0x253
 #define OPT_GPU_IDS 0x254
 #define OPT_RX_OFFSET 0x255
+#define OPT_RX_DEGLITCH 0x256
 
 static const struct option long_options[] = {
     { "rx", required_argument, 0, 'r' },
@@ -45,6 +48,7 @@ static const struct option long_options[] = {
     { "rx-filter", required_argument, 0, 'F' },
     { "rx-fmt", required_argument, 0, OPT_RX_FMT },
     { "rx-offset", required_argument, 0, OPT_RX_OFFSET },
+    { "rx-deglitch", required_argument, 0, OPT_RX_DEGLITCH },
     { "sdr-args", required_argument, 0, 'A' },
     { "frequency", required_argument, 0, 'f' },
     { "samplerate", required_argument, 0, 's' },
@@ -89,7 +93,11 @@ static void usage(const char *argv0)
     printf("  -B, --rx-rec-dig <filename>   Save the digital signal transitions to a CSV file.\n");
     printf("  --rx-fmt <fmt>                \"csv\" or \"pretty\" (default).\n");
     printf("  --rx-offset <Hz>              Decode a transmitter this far from the capture's centre frequency\n");
-    printf("                                (signed, K/M/G suffixes allowed; below half the sample rate).\n\n");
+    printf("                                (signed, K/M/G suffixes allowed; below half the sample rate).\n");
+    printf("  --rx-deglitch <n>|<t>us       Remove on/off runs of up to n outputs (or t microseconds) before the\n");
+    printf("                                state machine: each decision becomes the majority of the last 2n+1.\n");
+    printf("                                Delays every edge by n outputs.  0 (default): off; n <= %u.\n\n",
+           OOKD_DEGLITCH_MAX);
     printf("SDR configuration options:\n");
     printf("  -A, --sdr-args <file>         Capture file (\"-\": stdin): SC16Q11 for bladerf_file, interleaved\n");
     printf("                                uint8 I,Q for cu8_file, int8 I,Q for cs8_file.\n");
@@ -142,6 +150,29 @@ static bool parse_offset(const char *s, double *out)
     return isfinite(*out);
 }
 
+/* --rx-deglitch: <n> outputs (0 .. OOKD_DEGLITCH_MAX) or <t>us microseconds (converted once the decimation is known) */
+static bool parse_deglitch(const char *s, uint64_t *value, bool *in_us)
+{
+    if (!isdigit((unsigned char) s[0])) {
+        return false;
+    }
+    char *end;
+    errno = 0;
+    const unsigned long long v = strtoull(s, &end, 10);
+    if (errno) {
+        return false;
+    }
+    if (!strcmp(end, "us")) {
+        *in_us = true;
+    } else if (*end == '\0' && v <= OOKD_DEGLITCH_MAX) {
+        *in_us = false;
+    } else {
+        return false;
+    }
+    *value = v;
+    return true;
+}
+
 /* -T auto, -T auto:<dB>: a signed decimal margin over the median power */
 static bool parse_auto_threshold(const char *s, double *margin_db)
 {
@@ -181,6 +212,7 @@ int main(int argc, char *argv[])
     bool have_fmt = false;
     const char *offset_arg = NULL;
     double offset_hz = 0.0;
+    const char *deglitch_arg = NULL;
     int c, idx;
 
     ookd_cfg_init(&cfg);
@@ -297,6 +329,14 @@ int main(int argc, char *argv[])
                 }
                 offset_arg = optarg;
                 break;
+            case OPT_RX_DEGLITCH:
+                if (!parse_deglitch(optarg, &cfg.rx_deglitch, &cfg.rx_deglitch_us)) {
+                    fprintf(stderr, "Invalid RX deglitch: %s (a number of outputs from 0 to %u, or microseconds as "
+                            "<t>us)\n", optarg, OOKD_DEGLITCH_MAX);
+                    return EXIT_FAILURE;
+                }
+                deglitch_arg = optarg;
+                break;
             case 'A': cfg.sdr_args = optarg; break;
             case 's':
                 if (!parse_rate(optarg, &cfg.samplerate)) {
@@ -397,6 +437,10 @@ int main(int argc, char *argv[])
         }
         if (cfg.rx_threshold_auto) {
             fprintf(stderr, "Error: -T auto cannot be used with --tx.\n");
+            return EXIT_FAILURE;
+        }
+        if (deglitch_arg) {
+            fprintf(stderr, "Error: --rx-deglitch cannot be used with --tx.\n");
             return EXIT_FAILURE;
         }
         status = ookd_tx(&cfg);

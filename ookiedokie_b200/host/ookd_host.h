@@ -123,6 +123,10 @@ struct ookd_cfg {                       /* the fields of struct ookiedokie_cfg t
                                            OOKD_FLAG_INPUT_CU8 (cu8_file); recordings stay SC16Q11  */
     uint32_t tune_step;                 /* --rx-offset as ookd_gpu_config.tune_step (0: off); --rx-rec-input then
                                            records the tuned samples the decode saw                                */
+    uint64_t rx_deglitch;               /* --rx-deglitch: majority vote over 2M+1 decisions (ookd_gpu_config.deglitch),
+                                           M in outputs, or in microseconds with rx_deglitch_us; 0: off               */
+    bool     rx_deglitch_us;            /* ... converted with the decode's integer rate samplerate / decimation:
+                                           M = t * rate / 10^6 (u64), once the filter is loaded                      */
 };
 void ookd_cfg_init(struct ookd_cfg *cfg);               /* defaults of src/ookiedokie_cfg.c:27-38 */
 int  ookd_rx(const struct ookd_cfg *cfg);               /* 0 on success */

@@ -430,6 +430,24 @@ int ookd_rx(const struct ookd_cfg *cfg)
     gc.device_id = cfg->gpu_id;
     gc.flags = cfg->input_flags;
     gc.tune_step = cfg->tune_step;
+    if (cfg->rx_deglitch_us) {
+        /* microseconds at the state machine's integer rate (src/main.c:674-683) */
+        const uint64_t rate = cfg->samplerate / decimation;
+        if ((rate && cfg->rx_deglitch > UINT64_MAX / rate) || cfg->rx_deglitch * rate / 1000000 > OOKD_DEGLITCH_MAX) {
+            log_error("--rx-deglitch %" PRIu64 "us is more than %u outputs at %" PRIu64 " outputs/s.\n", cfg->rx_deglitch,
+                      OOKD_DEGLITCH_MAX, rate);
+            goto out;
+        }
+        gc.deglitch = (uint32_t) (cfg->rx_deglitch * rate / 1000000);
+    } else {
+        gc.deglitch = (uint32_t) cfg->rx_deglitch;
+    }
+    if (gc.deglitch) {
+        ookd_log(OOKD_LOG_INFO, "Deglitch: majority of %u decisions (runs of up to %u outputs removed)\n",
+                 2 * gc.deglitch + 1, gc.deglitch);
+    } else if (cfg->rx_deglitch_us) {
+        ookd_log(OOKD_LOG_INFO, "Deglitch: off (%" PRIu64 "us is less than one output)\n", cfg->rx_deglitch);
+    }
     const unsigned n_gpus = cfg->n_gpus > 1 ? cfg->n_gpus : 1;
     int rc;
     /* n_gpus > 1: one window over several GPUs, time shards with FIR halos, carries stitched on the host.  One GPU: two
